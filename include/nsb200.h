@@ -180,6 +180,32 @@ int nsb_get_coarse_operator(nsb_handle h, int64_t* n_rows, int64_t* n_blocks, in
  * bytes of the packed coarse operator, estimate of lambda_max(Dinv F) */
 int nsb_velocity_pc_info(nsb_handle h, int* two_level, int* smoother_degree, int* coarse_degree, int64_t* coarse_rows,
                          int64_t* coarse_value_bytes, double* fine_lambda_max);
+/* inspection (parity tests) of the velocity preconditioner's operators, one GPU only (an error with more ranks).  Vectors of a
+ * level are in its own global numbering: level 0 (fine) = the velocity DoFs, level 1 (coarse P1 level of the two-level cycle) =
+ * dim * vertex + component with vertex = pressure DoF - n_u.
+ *
+ * The packed copy of B = Dinv F of `level` exactly as the streamed operator reads it, unpacked from the tile headers, the quad
+ * metadata and the unique-neighbour lists into block CSR over the owned nodes: global node id of every row, block row pointer,
+ * global node id of every block column, dim*dim values per block (row-major, widened to double).  Also the level's stream
+ * tile count.  At precond_precision = 64 no copy is kept: precision 64 and no blocks.  NULL arrays are skipped (call once for
+ * the sizes). */
+int nsb_get_velocity_operator(nsb_handle h, int level, int* precision, int64_t* tiles, int64_t* n_rows, int64_t* n_blocks,
+                              int64_t* row_gid, int64_t* rowptr, int64_t* col_gid, double* vals);
+/* one application of the level's operator with the fused epilogue `mode` (coef = {cu, ct, cpu, cpy}):
+ *   2: y = B x ;  3: y = cu*u + ct*(B x), poly += cpu*u + cpy*y ;  4: y = cu*u + ct*(B x)
+ * u is read for modes 3 and 4, poly read and written for mode 3 (coef, u and poly may be NULL where unused). */
+int nsb_apply_velocity_operator(nsb_handle h, int level, int mode, const double coef[4], const double* x, const double* u, double* y,
+                                double* poly);
+/* roots of the level's polynomial as set up by the last nsb_solve, in application (Leja) order, one entry (re, im > 0) per
+ * conjugate pair; n = 0 for level 1 when the last setup chose the single-level polynomial.  NULL arrays are skipped. */
+int nsb_get_velocity_pc_roots(nsb_handle h, int level, int* n, double* re, double* im);
+/* the velocity preconditioner y_u ~ F^-1 x_u / the whole block preconditioner y = P^-1 x as set up by the last nsb_solve;
+ * x and y are global-length vectors (nsb_apply_velocity_pc reads and writes only their velocity entries) */
+int nsb_apply_velocity_pc(nsb_handle h, const double* x_global, double* y_global);
+int nsb_apply_preconditioner(nsb_handle h, const double* x_global, double* y_global);
+/* the Schur side of the block preconditioner: estimate of lambda_max(diag(M_p)^-1 M_p) that bounds its Jacobi-Chebyshev
+ * interval [1.1 lambda / 6, 1.1 lambda], and the coefficient of that M_p^-1 term (schur_mass_coeff resolved) */
+int nsb_pressure_pc_info(nsb_handle h, double* mp_lambda_max, double* mass_coeff);
 /* how many kernels this library launched since nsb_create */
 int nsb_launch_count(nsb_handle h, int64_t* n);
 

@@ -280,6 +280,56 @@ class Device:
         return dict(two_level=bool(a.value), smoother_degree=b.value, coarse_degree=d.value, coarse_rows=r.value,
                     coarse_value_bytes=v.value, fine_lambda_max=lm.value)
 
+    def velocity_operator(self, level):
+        """The packed B = Dinv F of `level` (0 fine, 1 coarse) as stored: dict(precision, tiles, row_gid, rowptr, col_gid,
+        vals[nblocks, dim, dim]) in the level's global node numbering."""
+        prec, nt, n, nb = C.c_int(), C.c_int64(), C.c_int64(), C.c_int64()
+        self._ck(lib().nsb_get_velocity_operator(self.h, level, C.byref(prec), C.byref(nt), C.byref(n), C.byref(nb),
+                                                 None, None, None, None))
+        rg, rp, cg = np.empty(n.value, np.int64), np.empty(n.value + 1, np.int64), np.empty(nb.value, np.int64)
+        v = np.empty((nb.value, self.dim, self.dim))
+        self._ck(lib().nsb_get_velocity_operator(self.h, level, C.byref(prec), C.byref(nt), C.byref(n), C.byref(nb),
+                                                 _p(rg, C.c_int64), _p(rp, C.c_int64), _p(cg, C.c_int64), _p(v, C.c_double)))
+        return dict(precision=prec.value, tiles=nt.value, row_gid=rg, rowptr=rp, col_gid=cg, vals=v)
+
+    def apply_velocity_operator(self, level, mode, x, u=None, poly=None, coef=(0.0, 0.0, 0.0, 0.0)):
+        """One application of the level's streamed operator with epilogue `mode` (2, 3, 4; coef = cu, ct, cpu, cpy) on
+        vectors in the level's global numbering.  Returns y, or (y, poly updated) for mode 3."""
+        x = np.ascontiguousarray(x, np.float64)
+        y = np.zeros_like(x)
+        cf = np.ascontiguousarray(coef, np.float64)
+        ua = None if u is None else np.ascontiguousarray(u, np.float64)
+        pa = None if poly is None else np.array(poly, np.float64)
+        self._ck(lib().nsb_apply_velocity_operator(self.h, level, mode, _p(cf, C.c_double), _p(x, C.c_double),
+                                                   None if ua is None else _p(ua, C.c_double), _p(y, C.c_double),
+                                                   None if pa is None else _p(pa, C.c_double)))
+        return (y, pa) if mode == 3 else y
+
+    def velocity_pc_roots(self, level):
+        """Roots of the level's polynomial (application order, one complex entry per conjugate pair)."""
+        n = C.c_int()
+        self._ck(lib().nsb_get_velocity_pc_roots(self.h, level, C.byref(n), None, None))
+        re, im = np.empty(n.value), np.empty(n.value)
+        self._ck(lib().nsb_get_velocity_pc_roots(self.h, level, C.byref(n), _p(re, C.c_double), _p(im, C.c_double)))
+        return re + 1j * im
+
+    def apply_velocity_pc(self, x):
+        x = np.ascontiguousarray(x, np.float64)
+        y = np.zeros(self.n_dofs)
+        self._ck(lib().nsb_apply_velocity_pc(self.h, _p(x, C.c_double), _p(y, C.c_double)))
+        return y
+
+    def apply_preconditioner(self, x):
+        x = np.ascontiguousarray(x, np.float64)
+        y = np.zeros(self.n_dofs)
+        self._ck(lib().nsb_apply_preconditioner(self.h, _p(x, C.c_double), _p(y, C.c_double)))
+        return y
+
+    def pressure_pc_info(self):
+        lm, cm = C.c_double(), C.c_double()
+        self._ck(lib().nsb_pressure_pc_info(self.h, C.byref(lm), C.byref(cm)))
+        return dict(mp_lambda_max=lm.value, mass_coeff=cm.value)
+
     def launch_count(self):
         n = C.c_int64()
         self._ck(lib().nsb_launch_count(self.h, C.byref(n)))

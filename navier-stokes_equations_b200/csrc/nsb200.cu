@@ -1055,6 +1055,11 @@ void amg_vcycle(nsb_ctx* c, int lev) {
 
 // ---- the block-triangular preconditioner (reference NavierStokes.hpp:320-344) -----------
 //   y0 = F~^-1 x0 ;  t = x1 - B y0 ;  y1 = -(rho/dt) Kp~^-1 t - cm Mp~^-1 t
+double schur_mass_coeff(const nsb_ctx* c) {
+  const double cm = c->opt.schur_mass_coeff;
+  return cm >= 0 ? cm : c->par.theta * c->par.nu + (c->par.use_supg ? c->par.gamma : 0.0);
+}
+
 void precond_apply(nsb_ctx* c, const double* x, double* y) {
   const Structure& S = c->S;
   const int dim = c->dim;
@@ -1087,8 +1092,7 @@ void precond_apply(nsb_ctx* c, const double* x, double* y) {
   amg_vcycle(c, 0);
   double* mres;
   csr_cheb(c, c->Mp, c->Mp_dinv.p, c->Mp_lmax, 6.0, c->opt.cheb_degree_Mp, tg, c->w_m0.p, c->w_m1.p, c->w_md.p, true, &mres);
-  double cm = c->opt.schur_mass_coeff;
-  if (cm < 0) cm = c->par.theta * c->par.nu + (c->par.use_supg ? c->par.gamma : 0.0);
+  const double cm = schur_mass_coeff(c);
   if (c->nranks > 1)
     k_lincomb_gather<<<nblk(S.np_own, 256), 256, 0, c->stream>>>(S.np_own, c->d_pid_gid.p, -(c->par.rho / c->par.dt), L0.x.p, -cm, mres, y + nu);
   else
@@ -1605,6 +1609,89 @@ double* vec_ptr(nsb_ctx* c, int which) {
     case NSB_RHS: return c->v_rhs.p;
   }
   return nullptr;
+}
+
+// ---- inspection of the velocity preconditioner's operators (parity tests) ------------------------------------------
+// Vectors of a level in its own global numbering: level 0 = velocity DoFs (dim * node + component), level 1 = the coarse
+// P1 level (dim * vertex + component, vertex = pressure DoF - n_u).  Level 1 is only mapped on one GPU (no ghost vertices).
+PolyLevel& level_of(nsb_ctx* c, int level) { return level == 0 ? c->lvF : c->lvC; }
+
+void level_upload(nsb_ctx* c, int level, const double* g, double* d) {
+  const Structure& S = c->S;
+  const int dim = c->dim;
+  const int nn = level == 0 ? S.nn_own + S.nn_ghost : S.np_own;
+  std::vector<double> loc(level == 0 ? (size_t)S.n_tot_dofs() : (size_t)dim * nn, 0.0);
+  for (int A = 0; A < nn; ++A) {
+    const int64_t off = level == 0 ? S.node_xoff(A) : (int64_t)dim * A;
+    const int64_t gid = level == 0 ? S.node_gid[A] : S.pid_gid[A];
+    for (int k = 0; k < dim; ++k) loc[off + k] = g[gid * dim + k];
+  }
+  CK(cudaMemcpyAsync(d, loc.data(), loc.size() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+}
+
+void level_download(nsb_ctx* c, int level, const double* d, double* g) {
+  const Structure& S = c->S;
+  const int dim = c->dim;
+  const int nn = level == 0 ? S.nn_own : S.np_own;
+  std::vector<double> out((size_t)dim * nn);
+  CK(cudaMemcpyAsync(out.data(), d, out.size() * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  for (int A = 0; A < nn; ++A) {
+    const int64_t gid = level == 0 ? S.node_gid[A] : S.pid_gid[A];
+    for (int k = 0; k < dim; ++k) g[gid * dim + k] = out[(size_t)dim * A + k];
+  }
+}
+
+// one level_apply<mode> on host vectors of the level's global numbering (u read for modes 3 / 4, poly read and written for 3)
+void velocity_operator_apply(nsb_ctx* c, int level, int mode, const double* coef, const double* xg, const double* ug, double* yg,
+                             double* pg) {
+  PolyLevel& lv = level_of(c, level);
+  double* x = level == 0 ? c->w_pin.p : c->cg.pin.p;
+  double* u = level == 0 ? c->w_u.p : c->cg.z0.p;
+  double* y = level == 0 ? c->w_tmp.p : c->cg.z1.p;
+  double* p = level == 0 ? c->w_poly.p : c->cg.poly.p;
+  level_upload(c, level, xg, x);
+  if (mode >= 3) level_upload(c, level, ug, u);
+  if (mode == 3) level_upload(c, level, pg, p);
+  const PolyCoef pc = coef ? PolyCoef{coef[0], coef[1], coef[2], coef[3]} : PolyCoef{};
+  if (mode == 2) level_apply<2>(c, lv, x, y, nullptr, nullptr, pc);
+  else if (mode == 3) level_apply<3>(c, lv, x, y, u, p, pc);
+  else level_apply<4>(c, lv, x, y, u, nullptr, pc);
+  level_download(c, level, y, yg);
+  if (mode == 3) level_download(c, level, p, pg);
+}
+
+// The packed copy of a level's B = Dinv F unpacked into (node, neighbour, dim*dim values) in stream order, from the tile
+// headers, the quad metadata and the unique-neighbour lists exactly as the streamed kernel reads them.
+template <typename VT>
+void unpack_level(nsb_ctx* c, const VsDev& D, int64_t total_nq, size_t n_uniq, std::vector<int>& node, std::vector<int>& nbr,
+                  std::vector<double>& val) {
+  const int dim = c->dim, PL = dim * dim;
+  std::vector<VsTile> tiles(D.n_tiles);
+  std::vector<uint32_t> meta((size_t)total_nq * 4);
+  std::vector<int> uniq(n_uniq);
+  std::vector<VT> v((size_t)total_nq * 4 * PL);
+  CK(cudaMemcpyAsync(tiles.data(), D.tiles, tiles.size() * sizeof(VsTile), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(meta.data(), D.meta, meta.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(uniq.data(), D.uniq_xoff, uniq.size() * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaMemcpyAsync(v.data(), D.vals, v.size() * sizeof(VT), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  for (const VsTile& T : tiles) {
+    const uint32_t* m = meta.data() + (size_t)T.nq_off * 4;
+    const VT* tv = v.data() + (size_t)T.nq_off * 4 * PL;
+    for (int q = 0; q < T.nquad; ++q) {
+      const uint32_t* mq = m + 4 * q;
+      if (mq[2] == 0xffffu) continue;
+      const int cnt = (int)(mq[3] >> 16);
+      for (int e = 0; e < cnt; ++e) {
+        const int loc = (int)(((e < 2 ? mq[0] : mq[1]) >> (16 * (e & 1))) & 0xffffu);
+        node.push_back(T.n0 + (int)mq[2]);
+        nbr.push_back(uniq[T.u0 + loc] / dim);
+        for (int rc = 0; rc < PL; ++rc) val.push_back((double)(float)tv[((size_t)rc * T.NQ + q) * 4 + e]);
+      }
+    }
+  }
 }
 
 }  // namespace
@@ -2182,20 +2269,122 @@ int nsb_apply_velocity_block(nsb_handle c, const double* xg, double* yg) {
   if (!c || !c->have_matrix) return fail(c, "no assembled system");
   NSB_TRY
   CK(cudaSetDevice(c->device));
-  const Structure& S = c->S;
-  std::vector<double> loc(S.n_tot_dofs(), 0.0);
-  const int dim = c->dim;
-  for (int A = 0; A < S.nn_own + S.nn_ghost; ++A)
-    for (int k = 0; k < dim; ++k) loc[S.node_xoff(A) + k] = xg[S.node_gid[A] * dim + k];
-  CK(cudaMemcpyAsync(c->w_pin.p, loc.data(), loc.size() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
-  spmv_vel<2>(c, c->w_pin.p, c->w_tmp.p, nullptr, nullptr, PolyCoef{});
-  std::vector<double> out((size_t)dim * S.nn_own);
-  CK(cudaMemcpyAsync(out.data(), c->w_tmp.p, out.size() * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
-  CK(cudaStreamSynchronize(c->stream));
-  for (int A = 0; A < S.nn_own; ++A)
-    for (int k = 0; k < dim; ++k) yg[S.node_gid[A] * dim + k] = out[(size_t)dim * A + k];
+  velocity_operator_apply(c, 0, 2, nullptr, xg, nullptr, yg, nullptr);     // the velocity block leads the global numbering
   return 0;
   NSB_CATCH(c)
+}
+
+// the checks shared by the inspection entries of one level
+static int level_entry_check(nsb_handle c, int level, const char* what) {
+  if (!c || !c->have_matrix) return fail(c, "no assembled system");
+  if (c->nranks > 1) return fail(c, std::string(what) + ": single GPU only (global numbering of one rank's vectors)");
+  if (level != 0 && level != 1) return fail(c, std::string(what) + ": level must be 0 (fine) or 1 (coarse)");
+  return 0;
+}
+
+int nsb_get_velocity_operator(nsb_handle c, int level, int* precision, int64_t* tiles, int64_t* n_rows, int64_t* n_blocks,
+                              int64_t* row_gid, int64_t* rowptr, int64_t* col_gid, double* vals) {
+  if (int rc = level_entry_check(c, level, "nsb_get_velocity_operator")) return rc;
+  NSB_TRY
+  CK(cudaSetDevice(c->device));
+  const Structure& S = c->S;
+  const int prec = c->opt.precond_precision, PL = c->dim * c->dim;
+  const int nn = level == 0 ? S.nn_own : S.np_own;
+  if (precision) *precision = prec;
+  if (tiles) *tiles = level == 0 ? c->n_stiles : c->cg.n_tiles;
+  if (n_rows) *n_rows = nn;
+  if (row_gid) for (int A = 0; A < nn; ++A) row_gid[A] = level == 0 ? S.node_gid[A] : S.pid_gid[A];
+  std::vector<int> node, nbr;
+  std::vector<double> v;
+  if (prec != 64) {
+    if (level == 0 && !c->vs_valid) return fail(c, "the packed velocity operator does not match the assembled system");
+    if (level == 1 && !c->cg.valid) return fail(c, "the coarse operator has not been assembled (linearised systems with velocity_cycle = 2 only)");
+    const VsDev D = level == 0 ? fine_dev(c) : coarse_dev(c);
+    const int64_t nq = level == 0 ? c->vs_total_nq : c->cg.total_nq;
+    const size_t nuq = level == 0 ? c->d_suniq_xoff.n : c->cg.uniq_xoff.n;
+    if (prec == 16) unpack_level<__half>(c, D, nq, nuq, node, nbr, v);
+    else unpack_level<float>(c, D, nq, nuq, node, nbr, v);
+  }
+  if (n_blocks) *n_blocks = (int64_t)node.size();
+  std::vector<int64_t> rp(nn + 1, 0);
+  for (int a : node) ++rp[a + 1];
+  for (int A = 0; A < nn; ++A) rp[A + 1] += rp[A];
+  if (rowptr) std::copy(rp.begin(), rp.end(), rowptr);
+  std::vector<int64_t> cur(rp.begin(), rp.end() - 1);
+  for (size_t i = 0; i < node.size(); ++i) {
+    const int64_t k = cur[node[i]]++;
+    if (col_gid) col_gid[k] = level == 0 ? S.node_gid[nbr[i]] : S.pid_gid[nbr[i]];
+    if (vals) std::copy(v.begin() + i * PL, v.begin() + (i + 1) * PL, vals + k * PL);
+  }
+  return 0;
+  NSB_CATCH(c)
+}
+
+int nsb_apply_velocity_operator(nsb_handle c, int level, int mode, const double coef[4], const double* x, const double* u, double* y,
+                                double* poly) {
+  if (int rc = level_entry_check(c, level, "nsb_apply_velocity_operator")) return rc;
+  if (mode < 2 || mode > 4) return fail(c, "nsb_apply_velocity_operator: mode must be 2, 3 or 4");
+  if (mode >= 3 && (!coef || !u || (mode == 3 && !poly))) return fail(c, "nsb_apply_velocity_operator: missing coefficients or vectors");
+  if (level == 1 && !c->cg.valid) return fail(c, "the coarse operator has not been assembled (linearised systems with velocity_cycle = 2 only)");
+  NSB_TRY
+  CK(cudaSetDevice(c->device));
+  velocity_operator_apply(c, level, mode, coef, x, u, y, poly);
+  return 0;
+  NSB_CATCH(c)
+}
+
+int nsb_get_velocity_pc_roots(nsb_handle c, int level, int* n, double* re, double* im) {
+  if (int rc = level_entry_check(c, level, "nsb_get_velocity_pc_roots")) return rc;
+  const auto& R = level_of(c, level).roots;
+  const size_t k = (level == 1 && !c->two_level) ? 0 : R.size();
+  if (n) *n = (int)k;
+  for (size_t i = 0; i < k; ++i) {
+    if (re) re[i] = R[i].first;
+    if (im) im[i] = R[i].second;
+  }
+  return 0;
+}
+
+// the preconditioner as set up by the last solve: it exists, and the two-level cycle's coarse operator is the current one
+static int pc_entry_check(nsb_handle c, const char* what) {
+  if (int rc = level_entry_check(c, 0, what)) return rc;
+  if (!c->have_pressure) return fail(c, "nsb_assemble_pressure_matrices has not been called");
+  if (c->lvF.roots.empty()) return fail(c, std::string(what) + ": no preconditioner has been set up (call nsb_solve first)");
+  if (c->two_level && !c->cg.valid) return fail(c, std::string(what) + ": the two-level cycle's coarse operator no longer matches the assembled system");
+  return 0;
+}
+
+int nsb_apply_velocity_pc(nsb_handle c, const double* xg, double* yg) {
+  if (int rc = pc_entry_check(c, "nsb_apply_velocity_pc")) return rc;
+  NSB_TRY
+  CK(cudaSetDevice(c->device));
+  const size_t n = (size_t)c->S.n_own_dofs(), nu = (size_t)c->dim * c->S.nn_own;      // one GPU: local layout == global numbering
+  CK(cudaMemcpyAsync(c->w_tmp.p, xg, n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+  apply_velocity_pc(c, c->w_tmp.p);
+  CK(cudaMemcpyAsync(yg, c->w_poly.p, nu * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return 0;
+  NSB_CATCH(c)
+}
+
+int nsb_apply_preconditioner(nsb_handle c, const double* xg, double* yg) {
+  if (int rc = pc_entry_check(c, "nsb_apply_preconditioner")) return rc;
+  NSB_TRY
+  CK(cudaSetDevice(c->device));
+  const size_t n = (size_t)c->S.n_own_dofs();
+  CK(cudaMemcpyAsync(c->w_tmp.p, xg, n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+  precond_apply(c, c->w_tmp.p, c->w_in.p);
+  CK(cudaMemcpyAsync(yg, c->w_in.p, n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return 0;
+  NSB_CATCH(c)
+}
+
+int nsb_pressure_pc_info(nsb_handle c, double* mp_lambda_max, double* mass_coeff) {
+  if (!c || !c->have_pressure) return fail(c, "pressure matrices not assembled");
+  if (mp_lambda_max) *mp_lambda_max = c->Mp_lmax;
+  if (mass_coeff) *mass_coeff = schur_mass_coeff(c);
+  return 0;
 }
 
 int nsb_timer_start(nsb_handle c) {

