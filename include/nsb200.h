@@ -124,6 +124,22 @@ int nsb_get_vector(nsb_handle h, int which, double* v_global);
 int nsb_copy_vector(nsb_handle h, int dst, int src);
 int nsb_axpy_vector(nsb_handle h, int dst, double alpha, int src);
 
+/* forcing term f of the momentum equation (reference NavierStokes.hpp:150-171), sampled by the caller at the
+ * quadrature points of the LOCAL cells (owned + ghost layer, nsb_get_sizes' n_cells_local).  The assembly uses
+ * f_theta = theta f(t) + (1 - theta) f(t - dt) in the rhs and in the SUPG source / strong residual
+ * (linearised system cpp:688-720, 733; Newton cpp:367-370, 488-506). */
+enum {
+  NSB_FORCING_NEW = 0,       /* f at t          */
+  NSB_FORCING_OLD = 1        /* f at t - dt     */
+};
+/* mapped quadrature points of the local cells, in the order nsb_set_forcing expects: pts[n_cells_local][n_q][dim],
+ * x_q = sum_v lambda_{q,v} X_v of QGaussSimplex<dim>(3) (n_q = 7 in 2-D, 10 in 3-D).  pts = NULL: n_q only. */
+int nsb_get_quadrature_points(nsb_handle h, int* n_q, double* pts);
+/* f[n_cells_local][n_q][dim], the forcing's velocity components at those points, into slot `which`; NULL or all zero
+ * clears the slot.  Both slots clear (the default) = no forcing: the kernels then read nothing and the assembled system
+ * is bit-identical to one that never had forcing.  Replaces the previous values of the slot; a new mesh clears both. */
+int nsb_set_forcing(nsb_handle h, int which, const double* f);
+
 /* ---- the hot path ----------------------------------------------------------------- */
 /* assemble_linearized_system()  (cpp:569-831): A, b from u^n, u^{n-1}, constraints, params */
 int nsb_assemble_linearized(nsb_handle h);

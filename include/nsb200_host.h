@@ -38,6 +38,7 @@ typedef struct nsh_options {
 typedef struct nsh_step_info {
   double time, cd, cl, dp, wall_seconds;
   int32_t gmres_iterations, newton_iterations, solves, converged;
+  double forcing_seconds;    /* host time of the step spent evaluating and uploading the forcing term */
 } nsh_step_info;
 
 const char* nsh_last_error(void);
@@ -54,6 +55,13 @@ int nsh_get_solution(nsh_handle h, double* current_solution /* [n_u+n_p] */);
 nsb_handle nsh_device(nsh_handle h);
 /* test hook, see nsh_options.test_fail_solves */
 int nsh_set_test_fail_solves(nsh_handle h, int32_t k);
+
+/* forcing term of the momentum equation (NavierStokes::set_forcing_term, reference hpp:150-171) as a batched callback:
+ * fn writes f(x_i, t) for the n points pts[n][dim] into out[n][dim] (velocity components) and returns 0; any other return
+ * value fails the step that asked for it.  The solver calls fn at most twice per assembly (t and t - dt), on the
+ * quadrature points of its local cells.  fn = NULL restores the default zero forcing. */
+typedef int (*nsh_forcing_fn)(int64_t n, const double* pts, double t, double* out, void* user);
+int nsh_set_forcing(nsh_handle h, nsh_forcing_fn fn, void* user);
 
 /* ---- host-only setup objects -------------------------------------------------------------- */
 int nshd_create(const char* mesh_file, int dim, nshd_handle* out);

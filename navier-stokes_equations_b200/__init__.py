@@ -17,6 +17,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("NSB200_LIB", os.path.join(_HERE, "libnsb200.so"))   # override: kernel-variant experiments
 
 NSB_SOLUTION_OLD, NSB_SOLUTION_OLD_OLD, NSB_CURRENT_SOLUTION, NSB_SOLUTION, NSB_RHS = 0, 1, 2, 3, 4
+NSB_FORCING_NEW, NSB_FORCING_OLD = 0, 1
 PROFILE_CLASSES = ("asm_context", "asm_rows", "spmv", "spmv_vel", "schur", "amg", "orth", "other", "asm_pack", "coarse", "asm_coarse")
 
 
@@ -169,6 +170,32 @@ class Device:
 
     def axpy_vector(self, dst, alpha, src):
         self._ck(lib().nsb_axpy_vector(self.h, dst, C.c_double(alpha), src))
+
+    def quadrature_points(self):
+        """Mapped quadrature points of the local cells, (n_cells_local, n_q, dim): where set_forcing's values belong."""
+        _, _, nc = self.sizes()
+        nq = C.c_int()
+        self._ck(lib().nsb_get_quadrature_points(self.h, C.byref(nq), None))
+        pts = np.empty((nc, nq.value, self.dim))
+        self._ck(lib().nsb_get_quadrature_points(self.h, C.byref(nq), _p(pts, C.c_double)))
+        return pts
+
+    def set_forcing(self, f_new, f_old=None):
+        """Forcing at t (f_new) and at t - dt (f_old, default: the same values) at quadrature_points(); None = zero."""
+        if f_old is None:
+            f_old = f_new
+        for which, f in ((NSB_FORCING_NEW, f_new), (NSB_FORCING_OLD, f_old)):
+            if f is None:
+                self._ck(lib().nsb_set_forcing(self.h, which, None))
+                continue
+            a = np.ascontiguousarray(f, np.float64)
+            _, _, nc = self.sizes()
+            if a.size != nc * (7 if self.dim == 2 else 10) * self.dim:
+                raise ValueError("forcing must have shape (n_cells_local, n_q, dim), got %s" % (a.shape,))
+            self._ck(lib().nsb_set_forcing(self.h, which, _p(a, C.c_double)))
+
+    def clear_forcing(self):
+        self.set_forcing(None, None)
 
     # ---- hot path
     def assemble_linearized(self):
@@ -351,7 +378,8 @@ class NshOptions(C.Structure):
 
 class NshStepInfo(C.Structure):
     _fields_ = [("time", C.c_double), ("cd", C.c_double), ("cl", C.c_double), ("dp", C.c_double), ("wall_seconds", C.c_double),
-                ("gmres_iterations", C.c_int32), ("newton_iterations", C.c_int32), ("solves", C.c_int32), ("converged", C.c_int32)]
+                ("gmres_iterations", C.c_int32), ("newton_iterations", C.c_int32), ("solves", C.c_int32), ("converged", C.c_int32),
+                ("forcing_seconds", C.c_double)]
 
 
 def hostlib():
@@ -364,6 +392,10 @@ def hostlib():
         _hostlib.nsh_last_error.restype = C.c_char_p
         _hostlib.nsh_device.restype = C.c_void_p
     return _hostlib
+
+
+# int fn(int64_t n, const double* pts, double t, double* out, void* user)   (nsh_forcing_fn)
+_FORCING_FN = C.CFUNCTYPE(C.c_int, C.c_int64, C.POINTER(C.c_double), C.c_double, C.POINTER(C.c_double), C.c_void_p)
 
 
 class _BorrowedDevice(Device):
@@ -392,6 +424,8 @@ class HostSolver:
         if L.nsh_create(case.encode(), mesh_file.encode(), C.byref(o), C.byref(self.h)) != 0:
             raise NsbError(L.nsh_last_error().decode())
         self.dim = 2 if case.startswith("2D") else 3
+        self._forcing_cb = None
+        self._forcing_error = None
 
     def _ck(self, rc):
         if rc != 0:
@@ -405,8 +439,34 @@ class HostSolver:
 
     def step(self):
         info = NshStepInfo()
-        self._ck(hostlib().nsh_step(self.h, C.byref(info)))
+        self._forcing_error = None
+        if hostlib().nsh_step(self.h, C.byref(info)) != 0:
+            msg = hostlib().nsh_last_error().decode()
+            raise NsbError(msg) from self._forcing_error
         return {k: getattr(info, k) for k, _ in NshStepInfo._fields_}
+
+    def set_forcing(self, fn):
+        """Forcing term f: fn(points (n, dim), t) -> (n, dim), called at most twice per assembly (t and t - dt) on the
+        quadrature points of the solver's local cells.  None restores the default zero forcing."""
+        if fn is None:
+            self._forcing_cb = None
+            self._ck(hostlib().nsh_set_forcing(self.h, None, None))
+            return
+        dim = self.dim
+
+        def cb(n, pts, t, out, user):
+            try:
+                x = np.ctypeslib.as_array(pts, shape=(n, dim)).copy() if n else np.empty((0, dim))
+                f = np.asarray(fn(x, t), dtype=np.float64).reshape(n, dim)
+                if n:
+                    np.ctypeslib.as_array(out, shape=(n, dim))[:] = f
+                return 0
+            except Exception as e:       # reported by step() as the cause of the failed step
+                self._forcing_error = e
+                return 1
+
+        self._forcing_cb = _FORCING_FN(cb)        # must outlive every step that may call it
+        self._ck(hostlib().nsh_set_forcing(self.h, self._forcing_cb, None))
 
     def set_test_fail_solves(self, k):
         self._ck(hostlib().nsh_set_test_fail_solves(self.h, int(k)))

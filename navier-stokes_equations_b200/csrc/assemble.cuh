@@ -7,7 +7,9 @@
 // Two passes, both deterministic and atomics-free (DESIGN.md "Assembly"):
 //   1. k_cell_context : one warp per cell.  Evaluates u^n, u^{n-1} (or u^k, p^k), u*, tau at the
 //      quadrature points, writes the cell's rhs vector and its context: for the linearised system
-//      the finished scalar block S_ab (CtxL, 1 KB), for Newton the per-point data (Ctx).
+//      the finished scalar block S_ab (CtxL, 1 KB), for Newton the per-point data (Ctx).  FORCED adds a
+//      user-supplied body force, given per (cell, quadrature point) at t and at t - dt (cpp:688-697, 367-370);
+//      the unforced instantiations read nothing extra and are the same code as without that option.
 //   2. k_node_rows    : one warp per OWNED P2 node.  Walks the node's cells in ascending order,
 //      computes the dim (+1) local matrix rows of that node exploiting the component-block
 //      structure  A[(a,c),(b,d)] = delta_cd S_ab + gamma G^{cd}_ab (+ T^{cd}_ab for Newton),
@@ -63,10 +65,11 @@ template <int DIM> struct QS {
 #ifndef NSB_CTX_MIN_CTAS
 #define NSB_CTX_MIN_CTAS 2
 #endif
-template <int DIM, bool NEWTON>
+template <int DIM, bool NEWTON, bool FORCED>
 __global__ void __launch_bounds__(ASM_WARPS * 32, NSB_CTX_MIN_CTAS)
 k_cell_context(DevMesh M, AsmParams P, const FeTables* __restrict__ gT, const double* __restrict__ vecA,
-               const double* __restrict__ vecB, double* __restrict__ ctx_out, double* __restrict__ cell_rhs) {
+               const double* __restrict__ vecB, double* __restrict__ ctx_out, double* __restrict__ cell_rhs,
+               const double* __restrict__ f_new, const double* __restrict__ f_old) {
   constexpr int NV = DIM + 1, NN = Fe<DIM>::NN, NQ = Fe<DIM>::NQ, DPC = Fe<DIM>::DPC;
   using C = Ctx<DIM>;
   using Q = QS<DIM>;
@@ -184,18 +187,34 @@ k_cell_context(DevMesh M, AsmParams P, const FeTables* __restrict__ gT, const do
       for (int k = 0; k < DIM; ++k) { t += gA[c][k] * ua[k]; if (NEWTON) r += gB[c][k] * ub[k]; }
       convA[c] = t; convB[c] = r;
     }
+    // forcing f_theta = theta f(t) + (1 - theta) f(t - dt) at this point ([cell][q][DIM], contiguous per cell); loaded
+    // here rather than at the top of phase B because the gradient accumulators are dead by now (no spills)
+    double fth[DIM];
+    if (FORCED) {
+      const size_t fo = ((size_t)cell * NQ + q) * DIM;
+#pragma unroll
+      for (int c = 0; c < DIM; ++c) fth[c] = P.theta * __ldg(f_new + fo + c) + (1.0 - P.theta) * __ldg(f_old + fo + c);
+    }
     if (!NEWTON) {
       // rhs of the linearised system (cpp:702-745)
 #pragma unroll
       for (int c = 0; c < DIM; ++c) {
         o[Q::M + c] = JxW * (P.inv_dt * ua[c] - (1.0 - P.theta) * convA[c]);
+        if (FORCED) o[Q::M + c] += JxW * fth[c];
         const double E = tw * ustar[c];                    // tau u*_c JxW: first-index contraction, cpp:733
 #pragma unroll
         for (int m = 0; m < NV; ++m) {
           double gg = 0, z = 0;
+          if (FORCED) {
+            // SUPG source with the same first-index contraction: tau u*_c grad phi_a . (f_theta + u^n / dt)   (cpp:733)
 #pragma unroll
-          for (int k = 0; k < DIM; ++k) { gg += gl[m][k] * gA[c][k]; z += gl[m][k] * ua[k]; }
-          o[Q::WZ + c * NV + m] = -JxW * (1.0 - P.theta) * P.nu * gg + E * (z * P.inv_dt);
+            for (int k = 0; k < DIM; ++k) { gg += gl[m][k] * gA[c][k]; z += gl[m][k] * (ua[k] * P.inv_dt + fth[k]); }
+            o[Q::WZ + c * NV + m] = -JxW * (1.0 - P.theta) * P.nu * gg + E * z;
+          } else {
+#pragma unroll
+            for (int k = 0; k < DIM; ++k) { gg += gl[m][k] * gA[c][k]; z += gl[m][k] * ua[k]; }
+            o[Q::WZ + c * NV + m] = -JxW * (1.0 - P.theta) * P.nu * gg + E * (z * P.inv_dt);
+          }
         }
       }
     } else {
@@ -224,7 +243,11 @@ k_cell_context(DevMesh M, AsmParams P, const FeTables* __restrict__ gT, const do
       for (int c = 0; c < DIM; ++c) {
         tr += gA[c][c];
         o[Q::M + c] = -JxW * ((ua[c] - ub[c]) * P.inv_dt + P.theta * convA[c] + (1.0 - P.theta) * convB[c]);
-        const double strong = (ua[c] - ub[c]) * P.inv_dt + convA[c] + gp[c] - P.nu * lap[c];
+        double strong = (ua[c] - ub[c]) * P.inv_dt + convA[c] + gp[c] - P.nu * lap[c];
+        if (FORCED) {
+          o[Q::M + c] += JxW * fth[c];
+          strong -= fth[c];                                // strong residual of the SUPG term (cpp:488-506)
+        }
 #pragma unroll
         for (int m = 0; m < NV; ++m) {
           double ga = 0, gb = 0;

@@ -295,6 +295,10 @@ struct nsb_ctx {
   nsb_params par{};
   nsb_solver_opts opt{};
   DBuf<double> vals, dinv, ctx, cell_rhs;
+  // forcing per (local cell, quadrature point, component) at t and t - dt (nsb_set_forcing): both allocated while either
+  // slot is non-zero, both freed when both are cleared; forcing_set[k] = slot k holds non-zero values
+  DBuf<double> forcing[2];
+  bool forcing_set[2] = {false, false};
   // streamed velocity operator (velstream.cuh): packed copy of Dinv F in fp32 / fp16, tile headers, block metadata
   DBuf<unsigned char> vs_vals;
   DBuf<VsTile> d_vs_tiles;
@@ -465,10 +469,16 @@ template <int DIM> void launch_assemble(nsb_ctx* c, bool newton) {
   const double* vecB = newton ? c->v_old.p : c->v_oldold.p;
   size_t id = c->prof.begin(PC_ASM_CTX, c->stream);
   const int cgrid = std::min(nblk(c->S.nc, ASM_WARPS), c->num_sms * 8);     // persistent: CTAs stride over the cells
-  if (newton)
-    k_cell_context<DIM, true><<<cgrid, ASM_WARPS * 32, 0, c->stream>>>(c->M, P, c->d_fe.p, vecA, vecB, c->ctx.p, c->cell_rhs.p);
+  const double *fn = c->forcing[NSB_FORCING_NEW].p, *fo = c->forcing[NSB_FORCING_OLD].p;
+  const bool forced = fn != nullptr;          // both slots are allocated together, and only while one is non-zero
+  if (newton && forced)
+    k_cell_context<DIM, true, true><<<cgrid, ASM_WARPS * 32, 0, c->stream>>>(c->M, P, c->d_fe.p, vecA, vecB, c->ctx.p, c->cell_rhs.p, fn, fo);
+  else if (newton)
+    k_cell_context<DIM, true, false><<<cgrid, ASM_WARPS * 32, 0, c->stream>>>(c->M, P, c->d_fe.p, vecA, vecB, c->ctx.p, c->cell_rhs.p, nullptr, nullptr);
+  else if (forced)
+    k_cell_context<DIM, false, true><<<cgrid, ASM_WARPS * 32, 0, c->stream>>>(c->M, P, c->d_fe.p, vecA, vecB, c->ctx.p, c->cell_rhs.p, fn, fo);
   else
-    k_cell_context<DIM, false><<<cgrid, ASM_WARPS * 32, 0, c->stream>>>(c->M, P, c->d_fe.p, vecA, vecB, c->ctx.p, c->cell_rhs.p);
+    k_cell_context<DIM, false, false><<<cgrid, ASM_WARPS * 32, 0, c->stream>>>(c->M, P, c->d_fe.p, vecA, vecB, c->ctx.p, c->cell_rhs.p, nullptr, nullptr);
   c->launch_check();
   c->prof.end(id, c->stream);
   RowOut out{c->vals.p, c->v_rhs.p, c->dinv.p};
@@ -1793,6 +1803,8 @@ int nsb_upload_mesh(nsb_handle c, int64_t n_vertices, const double* coords, int6
   if (!c) return -1;
   NSB_TRY
   CK(cudaSetDevice(c->device));
+  for (auto& b : c->forcing) b.alloc(0);    // forcing values belong to the previous mesh's local cells
+  c->forcing_set[0] = c->forcing_set[1] = false;
   const int dim = c->dim, NV = dim + 1;
   std::string e = build_structure(dim, n_vertices, coords, n_cells, cell_vertices, cell_dofs, n_u, n_p,
                                   c->nranks > 1 ? cell_part : nullptr, c->rank, c->nranks, c->S);
@@ -2043,6 +2055,58 @@ int nsb_set_vector(nsb_handle c, int which, const double* vg) {
   }
   CK(cudaMemcpyAsync(d, loc, (size_t)S.n_tot_dofs() * sizeof(double), cudaMemcpyHostToDevice, c->stream));
   CK(cudaStreamSynchronize(c->stream));
+  return 0;
+  NSB_CATCH(c)
+}
+
+int nsb_get_quadrature_points(nsb_handle c, int* n_q, double* pts) {
+  if (!c || !c->have_mesh) return fail(c, "nsb_get_quadrature_points: no mesh uploaded");
+  NSB_TRY
+  const Structure& S = c->S;
+  const int dim = c->dim, NV = dim + 1;
+  FeTables T;
+  fill_tables(dim, T);
+  if (n_q) *n_q = T.nq;
+  if (!pts) return 0;
+  const int nq = T.nq;
+#pragma omp parallel for schedule(static)
+  for (int cl = 0; cl < S.nc; ++cl) {
+    const uint32_t* cv = c->cell_vertices.data() + (size_t)S.cell_gid[cl] * NV;
+    for (int q = 0; q < nq; ++q)
+      for (int k = 0; k < dim; ++k) {
+        double x = 0.0;
+        for (int v = 0; v < NV; ++v) x += T.lam[q][v] * c->coords[(size_t)cv[v] * dim + k];
+        pts[((size_t)cl * nq + q) * dim + k] = x;
+      }
+  }
+  return 0;
+  NSB_CATCH(c)
+}
+
+int nsb_set_forcing(nsb_handle c, int which, const double* f) {
+  if (!c || !c->have_mesh) return fail(c, "nsb_set_forcing: no mesh uploaded");
+  if (which != NSB_FORCING_NEW && which != NSB_FORCING_OLD)
+    return fail(c, "nsb_set_forcing: which must be NSB_FORCING_NEW (0) or NSB_FORCING_OLD (1)");
+  NSB_TRY
+  CK(cudaSetDevice(c->device));
+  const size_t n = (size_t)c->S.nc * (c->dim == 2 ? Fe<2>::NQ : Fe<3>::NQ) * c->dim;
+  bool nonzero = false;
+  if (f)
+    for (size_t i = 0; i < n && !nonzero; ++i) nonzero = f[i] != 0.0;
+  if (nonzero) {
+    if (!c->forcing[0].p) {
+      for (auto& b : c->forcing) { b.alloc(n); b.zero(c->stream); }
+    }
+    CK(cudaMemcpyAsync(c->forcing[which].p, f, n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
+    CK(cudaStreamSynchronize(c->stream));       // f is the caller's pageable buffer
+  } else if (c->forcing_set[which] && c->forcing_set[1 - which]) {
+    c->forcing[which].zero(c->stream);
+  }
+  c->forcing_set[which] = nonzero;
+  if (!c->forcing_set[0] && !c->forcing_set[1] && c->forcing[0].p) {
+    CK(cudaStreamSynchronize(c->stream));       // an assembly may still read them
+    for (auto& b : c->forcing) b.alloc(0);
+  }
   return 0;
   NSB_CATCH(c)
 }

@@ -41,6 +41,12 @@ public:
   virtual void vector_value(const Point<dim>& p, Vector<double>& values) const {
     for (unsigned int c = 0; c < n_components; ++c) values[c] = value(p, c);
   }
+  // deal.II's batched evaluation: values[i] = vector_value(points[i]); values must hold points.size() vectors of
+  // n_components entries.  The forcing term is evaluated through this (once per assembly time level), so a class
+  // that can evaluate many points at once overrides it.
+  virtual void vector_value_list(const std::vector<Point<dim>>& points, std::vector<Vector<double>>& values) const {
+    for (std::size_t i = 0; i < points.size(); ++i) vector_value(points[i], values[i]);
+  }
   virtual void set_time(const double t) { time = t; }
   double get_time() const { return time; }
   const unsigned int n_components;

@@ -29,6 +29,42 @@ BenchmarkTestCase<3> make3(const std::string& n, const std::string& mesh, double
   if (n == "3D-2Z") return TestCases::make_3D_2Z(mesh, TimeScheme::CrankNicolson, NonlinearMethod::Linearized, dt);
   return TestCases::make_3D_3Z(mesh, TimeScheme::CrankNicolson, NonlinearMethod::Linearized, dt);
 }
+// Function<dim> over the C callback of nsh_set_forcing: vector_value_list makes one call for all points.
+template <int dim> class CallbackForcing : public Function<dim> {
+public:
+  CallbackForcing(nsh_forcing_fn fn_, void* user_) : Function<dim>(dim + 1), fn(fn_), user(user_) {}
+  double value(const Point<dim>& p, const unsigned int component) const override {
+    Vector<double> v(dim + 1);
+    vector_value(p, v);
+    return v[component];
+  }
+  void vector_value(const Point<dim>& p, Vector<double>& values) const override {
+    double x[3] = {0, 0, 0}, o[3] = {0, 0, 0};
+    for (int d = 0; d < dim; ++d) x[d] = p[d];
+    call(1, x, o);
+    for (int c = 0; c < dim; ++c) values[c] = o[c];
+    if (values.size() > (size_t)dim) values[dim] = 0.0;
+  }
+  void vector_value_list(const std::vector<Point<dim>>& points, std::vector<Vector<double>>& values) const override {
+    const size_t n = points.size();
+    std::vector<double> x(n * dim), o(n * dim, 0.0);
+    for (size_t i = 0; i < n; ++i)
+      for (int d = 0; d < dim; ++d) x[i * dim + d] = points[i][d];
+    call((int64_t)n, x.data(), o.data());
+    for (size_t i = 0; i < n; ++i) {
+      for (int c = 0; c < dim; ++c) values[i][c] = o[i * dim + c];
+      if (values[i].size() > (size_t)dim) values[i][dim] = 0.0;
+    }
+  }
+private:
+  void call(int64_t n, const double* x, double* o) const {
+    const int rc = fn(n, x, this->get_time(), o, user);
+    if (rc != 0)
+      throw std::runtime_error("forcing callback returned " + std::to_string(rc) + " at t = " + std::to_string(this->get_time()));
+  }
+  nsh_forcing_fn fn;
+  void* user;
+};
 }  // namespace
 
 struct nsh_solver {
@@ -96,7 +132,7 @@ int nsh_step(nsh_handle h, nsh_step_info* info) {
   if (info) {
     info->time = s.time; info->cd = s.cd; info->cl = s.cl; info->dp = s.dp; info->wall_seconds = s.wall_seconds;
     info->gmres_iterations = s.gmres_iterations; info->newton_iterations = s.newton_iterations;
-    info->solves = s.solves; info->converged = s.converged ? 1 : 0;
+    info->solves = s.solves; info->converged = s.converged ? 1 : 0; info->forcing_seconds = s.forcing_seconds;
   }
   return 0;
   NSH_CATCH
@@ -133,6 +169,15 @@ int nsh_set_test_fail_solves(nsh_handle h, int32_t k) {
   if (!h) return -1;
   if (h->dim == 2) h->s2->options.test_fail_solves = k; else h->s3->options.test_fail_solves = k;
   return 0;
+}
+
+int nsh_set_forcing(nsh_handle h, nsh_forcing_fn fn, void* user) {
+  if (!h) { g_err = "null handle"; return -1; }
+  NSH_TRY
+  if (h->dim == 2) h->s2->set_forcing_term(fn ? std::make_shared<CallbackForcing<2>>(fn, user) : nullptr);
+  else h->s3->set_forcing_term(fn ? std::make_shared<CallbackForcing<3>>(fn, user) : nullptr);
+  return 0;
+  NSH_CATCH
 }
 
 nsb_handle nsh_device(nsh_handle h) { return h->dim == 2 ? h->s2->device() : h->s3->device(); }

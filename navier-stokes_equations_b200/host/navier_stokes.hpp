@@ -87,6 +87,7 @@ struct StepInfo {
   double time = 0, cd = 0, cl = 0, dp = 0, wall_seconds = 0;
   int gmres_iterations = 0, newton_iterations = 0, solves = 0;
   bool converged = true;
+  double forcing_seconds = 0;     // host time spent evaluating and uploading the forcing term (part of wall_seconds)
 };
 
 template <int dim> class NavierStokes {
@@ -118,7 +119,10 @@ public:
 
   void set_inlet_velocity(std::shared_ptr<Function<dim>> f) { inlet_velocity = f; }
   void set_dirichlet_bc(std::shared_ptr<Function<dim>> f) { dirichlet_bc = f; }
-  void set_forcing_term(std::shared_ptr<Function<dim>> f) { forcing_term = f; }
+  void set_forcing_term(std::shared_ptr<Function<dim>> f) {
+    forcing_term = f ? f : std::make_shared<ForcingTerm<dim>>();
+    forcing_time[0] = forcing_time[1] = std::nan("");
+  }
   void set_initial_condition(std::shared_ptr<Function<dim>> f) { initial_condition = f; }
 
   void setup();
@@ -191,10 +195,15 @@ protected:
   unsigned int time_step_no = 0;
   int last_gmres_iterations = 0, step_gmres_iterations = 0, step_solves = 0;
   double last_rhs_norm = 0.0;
-  mutable double forcing_checked_time = -1.0;
+  double step_forcing_seconds = 0.0;
+  // forcing uploaded to the device: the time each slot (NSB_FORCING_NEW / _OLD) was evaluated at, NaN = not uploaded
+  double forcing_time[2] = {std::nan(""), std::nan("")};
+  bool forcing_on_device = false;
+  std::vector<Point<dim>> forcing_points;      // quadrature points of the device's local cells (nsb_get_quadrature_points)
+  std::vector<Vector<double>> forcing_values;  // vector_value_list output, kept between evaluations
 
   void push_params(bool first_order);
-  void require_zero_forcing() const;
+  void update_forcing();
   void build_system_constraints();
   void ck(int rc, const char* what) const;
   std::function<double(const double*, int)> eval(const std::shared_ptr<Function<dim>>& f) const;

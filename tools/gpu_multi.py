@@ -2,9 +2,11 @@
 assembled matrix / rhs against the oracle and -- bit for bit -- against a single-GPU assembly of the same system,
 the tight-tolerance solve against a sparse direct solve, the iteration count at the reference tolerance
 (partition-independent preconditioner), and three time steps of the C++ host class NavierStokes<3>(make_3D_2Z)
-(BASELINE config 3, "1 vs 2 GPUs") with per-rank VTU pieces.
-  python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/gpu_multi.py [--json out.json]
-tests/test_gpu_multirank.py runs this under pytest and asserts on the JSON."""
+(BASELINE config 3, "1 vs 2 GPUs") with per-rank VTU pieces.  --forcing adds a body force everywhere: each rank
+samples it at its own local cells' quadrature points (owned + ghost layer), the oracle at its own, and the host class
+takes it through HostSolver.set_forcing.
+  python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/gpu_multi.py [--json out.json] [--forcing]
+tests/test_gpu_multirank.py and tests/test_gpu_forcing.py run this under pytest and assert on the JSON."""
 import argparse
 import json
 import os
@@ -22,6 +24,7 @@ import torch.distributed as dist  # noqa: E402
 from oracle import assemble as asm, dofs as odofs, postprocess as pp, solve as osolve  # noqa: E402
 import nsb200 as nsb  # noqa: E402
 from tests.conftest import synthetic_state  # noqa: E402
+from tests.forcing_cases import ForcedOracle, quadrature_points, sample, smooth_forcing  # noqa: E402
 from tools import meshgen, msh  # noqa: E402
 
 
@@ -30,6 +33,7 @@ def main():
     ap.add_argument("--json", default=None)
     ap.add_argument("--lc", type=float, default=0.04)
     ap.add_argument("--part", default="chunks", help="cell partition: chunks (contiguous) or metis (face-dual graph, like the reference)")
+    ap.add_argument("--forcing", action="store_true", help="assemble and step with a non-zero body force")
     args = ap.parse_args()
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
@@ -44,13 +48,21 @@ def main():
     con = odofs.build_constraints(mesh, dm, pp.inlet_profile(3, tc["U_m"], False, 4.0, 1.0), pp.boundary_ids(3))
     un, unm1 = synthetic_state(dm, 3, tc["U_m"])
     p = asm.Params(dt=0.01, theta=0.5, nu=1e-3, use_supg=True)
-    ref = asm.assemble(mesh, dm, pat, p, con, "linearized", un, unm1) if rank == 0 else None
+    t_new, t_old = 1.0, 0.99
+    forcing = None
+    if args.forcing:
+        qp = quadrature_points(mesh)
+        forcing = (sample(smooth_forcing, qp, t_new), sample(smooth_forcing, qp, t_old))
+    ref = asm.assemble(mesh, dm, pat, p, con, "linearized", un, unm1, forcing=forcing) if rank == 0 else None
     holder2 = [ref]
     dist.broadcast_object_list(holder2, src=0)
     ref = holder2[0]
 
     def setup(dev, part):
         dev.upload_mesh(mesh.points, mesh.cells, dm.cell_dofs, dm.n_u, dm.n_p, part)
+        if args.forcing:
+            qd = dev.quadrature_points()
+            dev.set_forcing(sample(smooth_forcing, qd, t_new), sample(smooth_forcing, qd, t_old))
         dev.set_constraints(con.dofs, con.val[con.dofs])
         dev.set_params(0.01, 0.5, 1e-3, 1.0, 0.1, True, False)
         dev.set_vector(nsb.NSB_SOLUTION_OLD, un)
@@ -118,11 +130,13 @@ def main():
     dist.broadcast_object_list(holder3, src=0)
     hs = nsb.HostSolver("3D-2Z", path, device=local, rank=rank, nranks=world, nccl_unique_id=holder3[0], gmres_tolerance=1e-12,
                         write_vtu=True, output_dir=outdir, partitioner=1 if args.part == "metis" else 0)
+    if args.forcing:
+        hs.set_forcing(smooth_forcing)
     hs.initialize()
     infos = [hs.step() for _ in range(3)]
     steps = []
     if rank == 0:
-        o = osolve.Oracle(mesh, "3D-2Z", solver="direct")
+        o = ForcedOracle(mesh, "3D-2Z", smooth_forcing, solver="direct") if args.forcing else osolve.Oracle(mesh, "3D-2Z", solver="direct")
         for k, info in enumerate(infos):
             ref_ = o.step()
             errs = {key: abs(info[key] - ref_[key]) / max(abs(ref_[key]), 1e-300) for key in ("cd", "cl", "dp")}
@@ -142,7 +156,7 @@ def main():
         for src in pieces:
             piece = ET.parse(outdir + src).getroot().find("UnstructuredGrid/Piece")
             ncell += int(piece.get("NumberOfCells"))
-        summary = dict(world=world, partition=args.part, fused=os.environ.get("NSB200_FUSED_HALO", "0"), halo=os.environ.get("NSB200_HALO", "p2p"), mesh_cells=int(mesh.n_cells), n_dofs=int(N),
+        summary = dict(world=world, partition=args.part, forcing=bool(args.forcing), fused=os.environ.get("NSB200_FUSED_HALO", "0"), halo=os.environ.get("NSB200_HALO", "p2p"), mesh_cells=int(mesh.n_cells), n_dofs=int(N),
                        ranks=recs, host_class_steps=steps, host_class_field_relerr=field, vtu_pieces=pieces, vtu_cells_total=ncell)
         print("[summary] " + json.dumps(summary), flush=True)
         if args.json:
