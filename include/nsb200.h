@@ -140,6 +140,35 @@ int nsb_get_quadrature_points(nsb_handle h, int* n_q, double* pts);
  * is bit-identical to one that never had forcing.  Replaces the previous values of the slot; a new mesh clears both. */
 int nsb_set_forcing(nsb_handle h, int which, const double* f);
 
+/* Forcing evaluated on the device from CUDA source compiled at run time (NVRTC, loaded on first use; without it only these
+ * entries fail).  The source defines a function named nsb_forcing with this signature (the library checks it exactly):
+ *     __device__ void <nsb_forcing>(const double* x, double t, const double* prm, double* f);
+ * x[NSB_DIM] is a quadrature point, prm[] the parameters passed here, f[NSB_DIM] the velocity components (zeroed before the
+ * call).  The library puts `#define NSB_DIM 2|3` before the text and its evaluation kernel after it.  No #include; NVRTC's
+ * built-in math (sin, cos, exp, pow, sqrt, ...) is available, M_PI is not defined; helper __device__ functions and constants
+ * may be defined.  Compiled with --gpu-architecture=sm_XYa of the handle's device and -std=c++17.
+ *
+ * Compiles `src` (or reuses the kernel when the text equals the one already loaded: nothing is compiled) and stores
+ * prm[n_prm], 0 <= n_prm <= 16 (prm may be NULL when n_prm = 0).  A compile error returns < 0 and nsb_last_error carries
+ * NVRTC's log, whose line numbers count the lines of `src`.  On first use the local cells' vertex coordinates and cell ->
+ * vertex table are copied to the device (freed by a new mesh).  The slots keep their values until the next
+ * nsb_eval_forcing / nsb_set_forcing.  src = NULL unloads the kernel and clears both slots.  Errors: no mesh uploaded,
+ * n_prm out of range, prm = NULL with n_prm > 0. */
+int nsb_set_forcing_source(nsb_handle h, const char* src, const double* prm, int n_prm);
+/* fills slot `which` on the device with f(x_q, t) at the points of nsb_get_quadrature_points (mapped on the device with
+ * the same operations in the same order: bit-identical points).  An all-zero result clears the slot as nsb_set_forcing
+ * does.  Synchronises (reads back 4 bytes).  A later nsb_set_forcing of the slot replaces its values, and vice versa.
+ * Errors: no mesh uploaded, bad `which`, no source set. */
+int nsb_eval_forcing(nsb_handle h, int which, double t);
+/* inspection: slot `which` as f[n_cells_local][n_q][dim]; returns 1 (soft) and zeros when the slot is clear */
+int nsb_get_forcing(nsb_handle h, int which, double* f);
+/* a source is loaded; sources compiled and slots evaluated since nsb_create; version of the NVRTC that was loaded
+ * (0.0 when none could be).  NULL pointers are skipped. */
+int nsb_forcing_info(nsb_handle h, int* has_source, int64_t* compiles, int64_t* evaluations, int* nvrtc_major, int* nvrtc_minor);
+/* compiles a forcing source for sm_100a without a handle or a GPU: 0 when it compiles, else < 0 with the error (NVRTC's log)
+ * in log[log_size] (truncated, NUL-terminated; log may be NULL) */
+int nsb_check_forcing_source(int dim, const char* src, char* log, size_t log_size);
+
 /* ---- the hot path ----------------------------------------------------------------- */
 /* assemble_linearized_system()  (cpp:569-831): A, b from u^n, u^{n-1}, constraints, params */
 int nsb_assemble_linearized(nsb_handle h);
@@ -173,7 +202,7 @@ int nsb_timer_start(nsb_handle h);
 int nsb_timer_stop(nsb_handle h, double* milliseconds);
 int nsb_synchronize(nsb_handle h);
 /* per-kernel-class CUDA-event profile: names "asm_context","asm_rows","spmv","spmv_vel",
- * "schur","amg","orth","other","asm_pack","coarse","asm_coarse" */
+ * "schur","amg","orth","other","asm_pack","coarse","asm_coarse","forcing" */
 int nsb_profile_enable(nsb_handle h, int on);
 int nsb_profile_reset(nsb_handle h);
 int nsb_profile_get(nsb_handle h, const char* name, double* total_ms, int64_t* launches);

@@ -38,7 +38,8 @@ typedef struct nsh_options {
 typedef struct nsh_step_info {
   double time, cd, cl, dp, wall_seconds;
   int32_t gmres_iterations, newton_iterations, solves, converged;
-  double forcing_seconds;    /* host time of the step spent evaluating and uploading the forcing term */
+  double forcing_seconds;    /* time of the step spent evaluating the forcing term and getting it to the device (host
+                                evaluation + upload, or device evaluation + synchronise for a forcing source) */
 } nsh_step_info;
 
 const char* nsh_last_error(void);
@@ -62,6 +63,11 @@ int nsh_set_test_fail_solves(nsh_handle h, int32_t k);
  * quadrature points of its local cells.  fn = NULL restores the default zero forcing. */
 typedef int (*nsh_forcing_fn)(int64_t n, const double* pts, double t, double* out, void* user);
 int nsh_set_forcing(nsh_handle h, nsh_forcing_fn fn, void* user);
+/* forcing term as CUDA source evaluated on the device (DeviceForcing; source contract and parameters as for
+ * nsb_set_forcing_source, at most 16).  The solver compiles it on the first step that needs it (a compile error fails that
+ * step with NVRTC's log) and evaluates each time level once per assembly time.  src = NULL restores the default zero
+ * forcing. */
+int nsh_set_forcing_source(nsh_handle h, const char* src, const double* prm, int32_t n_prm);
 
 /* ---- host-only setup objects -------------------------------------------------------------- */
 int nshd_create(const char* mesh_file, int dim, nshd_handle* out);

@@ -18,7 +18,7 @@ LIB_PATH = os.environ.get("NSB200_LIB", os.path.join(_HERE, "libnsb200.so"))   #
 
 NSB_SOLUTION_OLD, NSB_SOLUTION_OLD_OLD, NSB_CURRENT_SOLUTION, NSB_SOLUTION, NSB_RHS = 0, 1, 2, 3, 4
 NSB_FORCING_NEW, NSB_FORCING_OLD = 0, 1
-PROFILE_CLASSES = ("asm_context", "asm_rows", "spmv", "spmv_vel", "schur", "amg", "orth", "other", "asm_pack", "coarse", "asm_coarse")
+PROFILE_CLASSES = ("asm_context", "asm_rows", "spmv", "spmv_vel", "schur", "amg", "orth", "other", "asm_pack", "coarse", "asm_coarse", "forcing")
 
 
 class NsbError(RuntimeError):
@@ -53,6 +53,13 @@ def lib():
 
 def _p(a, ctype):
     return a.ctypes.data_as(C.POINTER(ctype))
+
+
+def check_forcing_source(dim, src):
+    """Compile a forcing source for sm_100a without a GPU (nsb_check_forcing_source); raises NsbError with NVRTC's log."""
+    buf = C.create_string_buffer(1 << 16)
+    if lib().nsb_check_forcing_source(int(dim), src.encode(), buf, C.c_size_t(len(buf))) != 0:
+        raise NsbError(buf.value.decode())
 
 
 class Device:
@@ -196,6 +203,31 @@ class Device:
 
     def clear_forcing(self):
         self.set_forcing(None, None)
+
+    def set_forcing_source(self, src, params=()):
+        """Forcing as CUDA source evaluated on the device (nsb_set_forcing_source): `src` defines
+        __device__ void nsb_forcing(const double* x, double t, const double* prm, double* f); params (at most 16) arrive as
+        prm.  Compiles unless the same source is already loaded.  None unloads it and clears both slots."""
+        prm = np.ascontiguousarray(params, np.float64).ravel()
+        self._ck(lib().nsb_set_forcing_source(self.h, None if src is None else src.encode(),
+                                              _p(prm, C.c_double) if prm.size else None, int(prm.size)))
+
+    def eval_forcing(self, which, t):
+        """Fill slot `which` (NSB_FORCING_NEW / NSB_FORCING_OLD) with the source's f at time t on the device."""
+        self._ck(lib().nsb_eval_forcing(self.h, which, C.c_double(t)))
+
+    def forcing(self, which):
+        """Slot `which` as (n_cells_local, n_q, dim); all zeros when the slot is clear."""
+        _, _, nc = self.sizes()
+        f = np.empty((nc, 7 if self.dim == 2 else 10, self.dim))
+        self._ck(lib().nsb_get_forcing(self.h, which, _p(f, C.c_double)), soft=(1,))
+        return f
+
+    def forcing_info(self):
+        hs, nv_maj, nv_min = C.c_int(), C.c_int(), C.c_int()
+        comp, ev = C.c_int64(), C.c_int64()
+        self._ck(lib().nsb_forcing_info(self.h, C.byref(hs), C.byref(comp), C.byref(ev), C.byref(nv_maj), C.byref(nv_min)))
+        return dict(has_source=bool(hs.value), compiles=comp.value, evaluations=ev.value, nvrtc=(nv_maj.value, nv_min.value))
 
     # ---- hot path
     def assemble_linearized(self):
@@ -467,6 +499,14 @@ class HostSolver:
 
         self._forcing_cb = _FORCING_FN(cb)        # must outlive every step that may call it
         self._ck(hostlib().nsh_set_forcing(self.h, self._forcing_cb, None))
+
+    def set_forcing_source(self, src, params=()):
+        """Forcing term as CUDA source evaluated on the GPU (DeviceForcing; see Device.set_forcing_source for the contract).
+        A compile error fails the first step that needs the forcing.  None restores the default zero forcing."""
+        prm = np.ascontiguousarray(params, np.float64).ravel()
+        self._forcing_cb = None
+        self._ck(hostlib().nsh_set_forcing_source(self.h, None if src is None else src.encode(),
+                                                  _p(prm, C.c_double) if prm.size else None, int(prm.size)))
 
     def set_test_fail_solves(self, k):
         self._ck(hostlib().nsh_set_test_fail_solves(self.h, int(k)))

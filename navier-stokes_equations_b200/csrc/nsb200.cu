@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 #include <dlfcn.h>
 #include <nccl.h>   // types only: the library is resolved at run time (see NcclApi)
+#include <nvrtc.h>  // types only: the library is resolved at run time (see NvrtcApi)
 
 #include <algorithm>
 #include <cmath>
@@ -84,6 +85,99 @@ struct NcclApi {
 };
 NcclApi g_nccl;
 
+// NVRTC compiles a user's device-side forcing term (nsb_set_forcing_source).  Bound lazily like NCCL: libnsb200.so has no
+// link-time dependency on it, and inside a PyTorch process the NVRTC torch already loaded may be the one found (any 12.8+
+// compiles for sm_100a; nsb_forcing_info reports the version).  Only the forcing-source entries need it.
+struct NvrtcApi {
+  void* handle = nullptr;
+  std::string err;
+  int major = 0, minor = 0;
+  const char* (*GetErrorString)(nvrtcResult) = nullptr;
+  nvrtcResult (*Version)(int*, int*) = nullptr;
+  nvrtcResult (*CreateProgram)(nvrtcProgram*, const char*, const char*, int, const char* const*, const char* const*) = nullptr;
+  nvrtcResult (*CompileProgram)(nvrtcProgram, int, const char* const*) = nullptr;
+  nvrtcResult (*GetProgramLogSize)(nvrtcProgram, size_t*) = nullptr;
+  nvrtcResult (*GetProgramLog)(nvrtcProgram, char*) = nullptr;
+  nvrtcResult (*GetCUBINSize)(nvrtcProgram, size_t*) = nullptr;
+  nvrtcResult (*GetCUBIN)(nvrtcProgram, char*) = nullptr;
+  nvrtcResult (*DestroyProgram)(nvrtcProgram*) = nullptr;
+  bool load() {
+    if (handle) return true;
+    if (!err.empty()) return false;
+    for (const char* name : {"libnvrtc.so.12", "libnvrtc.so"}) {
+      handle = dlopen(name, RTLD_NOW | RTLD_GLOBAL);
+      if (handle) break;
+    }
+    if (!handle) { err = std::string("cannot load NVRTC (libnvrtc.so.12), needed to compile a forcing source: ") + dlerror(); return false; }
+    auto sym = [&](const char* n) { void* p = dlsym(handle, n); if (!p) err = std::string("NVRTC symbol missing: ") + n; return p; };
+    GetErrorString = (decltype(GetErrorString))sym("nvrtcGetErrorString");
+    Version = (decltype(Version))sym("nvrtcVersion");
+    CreateProgram = (decltype(CreateProgram))sym("nvrtcCreateProgram");
+    CompileProgram = (decltype(CompileProgram))sym("nvrtcCompileProgram");
+    GetProgramLogSize = (decltype(GetProgramLogSize))sym("nvrtcGetProgramLogSize");
+    GetProgramLog = (decltype(GetProgramLog))sym("nvrtcGetProgramLog");
+    GetCUBINSize = (decltype(GetCUBINSize))sym("nvrtcGetCUBINSize");
+    GetCUBIN = (decltype(GetCUBIN))sym("nvrtcGetCUBIN");
+    DestroyProgram = (decltype(DestroyProgram))sym("nvrtcDestroyProgram");
+    if (!err.empty()) { dlclose(handle); handle = nullptr; return false; }
+    Version(&major, &minor);
+    return true;
+  }
+};
+NvrtcApi g_nvrtc;
+
+// csrc/forcing_eval.cuh as text (the Makefile wraps it in a raw string literal)
+const char kForcingEvalSrc[] =
+#include "../forcing_eval_src.inc"
+    ;
+
+constexpr int kForcingMaxParams = 16;
+constexpr int kForcingBlock = 256;
+
+// The NVRTC program for a forcing source: NSB_DIM / NSB_NQ, the user's text, the evaluation kernel.  The #line directives
+// make the compiler's messages name the user's lines as they wrote them.
+std::string forcing_program(int dim, const char* src, const std::string& opts) {
+  std::string p = "// device-side forcing term of nsb200, compiled with NVRTC: " + opts + "\n";
+  p += "#define NSB_DIM " + std::to_string(dim) + "\n#define NSB_NQ " + std::to_string(dim == 2 ? Fe<2>::NQ : Fe<3>::NQ) + "\n";
+  p += "#line 1 \"nsb_forcing.cu\"\n";
+  p += src;
+  p += "\n#line 1 \"forcing_eval.cuh\"\n";
+  p += kForcingEvalSrc;
+  return p;
+}
+
+// Compiles the forcing program for `arch` (e.g. "sm_100a").  Returns "" and the cubin, or the error with NVRTC's log.
+std::string compile_forcing(int dim, const char* src, const std::string& arch, std::vector<char>& cubin) {
+  if (!g_nvrtc.load()) return g_nvrtc.err;
+  const std::string o_arch = "--gpu-architecture=" + arch, o_std = "-std=c++17";
+  const char* opts[] = {o_arch.c_str(), o_std.c_str()};
+  const std::string text = forcing_program(dim, src, o_arch + " " + o_std);
+  nvrtcProgram prog;
+  nvrtcResult r = g_nvrtc.CreateProgram(&prog, text.c_str(), "nsb_forcing.cu", 0, nullptr, nullptr);
+  if (r != NVRTC_SUCCESS) return std::string("nvrtcCreateProgram failed: ") + g_nvrtc.GetErrorString(r);
+  r = g_nvrtc.CompileProgram(prog, 2, opts);
+  std::string msg;
+  if (r != NVRTC_SUCCESS) {
+    size_t n = 0;
+    g_nvrtc.GetProgramLogSize(prog, &n);
+    std::string log(n, '\0');
+    if (n) g_nvrtc.GetProgramLog(prog, &log[0]);
+    while (!log.empty() && (log.back() == '\0' || log.back() == '\n')) log.pop_back();
+    msg = std::string("forcing source does not compile (") + g_nvrtc.GetErrorString(r) + ", NVRTC " + std::to_string(g_nvrtc.major) +
+          "." + std::to_string(g_nvrtc.minor) + ", " + arch + "):\n" + log;
+  } else {
+    size_t n = 0;
+    r = g_nvrtc.GetCUBINSize(prog, &n);
+    if (r == NVRTC_SUCCESS) {
+      cubin.resize(n);
+      r = g_nvrtc.GetCUBIN(prog, cubin.data());
+    }
+    if (r != NVRTC_SUCCESS) msg = std::string("nvrtcGetCUBIN failed: ") + g_nvrtc.GetErrorString(r);
+  }
+  g_nvrtc.DestroyProgram(&prog);
+  return msg;
+}
+
 template <typename T> struct DBuf {
   T* p = nullptr;
   size_t n = 0;
@@ -110,8 +204,8 @@ template <typename T> struct DBuf {
   }
 };
 
-enum ProfCat { PC_ASM_CTX = 0, PC_ASM_ROWS, PC_SPMV, PC_SPMV_VEL, PC_SCHUR, PC_AMG, PC_ORTH, PC_OTHER, PC_ASM_PACK, PC_COARSE, PC_ASM_COARSE, PC_N };
-const char* kProfNames[PC_N] = {"asm_context", "asm_rows", "spmv", "spmv_vel", "schur", "amg", "orth", "other", "asm_pack", "coarse", "asm_coarse"};
+enum ProfCat { PC_ASM_CTX = 0, PC_ASM_ROWS, PC_SPMV, PC_SPMV_VEL, PC_SCHUR, PC_AMG, PC_ORTH, PC_OTHER, PC_ASM_PACK, PC_COARSE, PC_ASM_COARSE, PC_FORCING, PC_N };
+const char* kProfNames[PC_N] = {"asm_context", "asm_rows", "spmv", "spmv_vel", "schur", "amg", "orth", "other", "asm_pack", "coarse", "asm_coarse", "forcing"};
 
 struct Prof {
   bool on = false;
@@ -299,6 +393,17 @@ struct nsb_ctx {
   // slot is non-zero, both freed when both are cleared; forcing_set[k] = slot k holds non-zero values
   DBuf<double> forcing[2];
   bool forcing_set[2] = {false, false};
+  // device-evaluated forcing (nsb_set_forcing_source): the loaded evaluation kernel and the source it was compiled from,
+  // its parameters, and what it maps the quadrature points from -- the coordinates of the vertices of the local cells and
+  // a local cell -> vertex table (uploaded on first use, freed with the mesh)
+  cudaLibrary_t fsrc_lib = nullptr;
+  cudaKernel_t fsrc_kernel = nullptr;
+  std::string fsrc_text;
+  DBuf<double> fsrc_prm, fsrc_coords;
+  DBuf<int> fsrc_cells;
+  DBuf<unsigned int> fsrc_flag;
+  bool fsrc_geom = false;
+  int64_t fsrc_compiles = 0, fsrc_evals = 0;
   // streamed velocity operator (velstream.cuh): packed copy of Dinv F in fp32 / fp16, tile headers, block metadata
   DBuf<unsigned char> vs_vals;
   DBuf<VsTile> d_vs_tiles;
@@ -1704,6 +1809,58 @@ void unpack_level(nsb_ctx* c, const VsDev& D, int64_t total_nq, size_t n_uniq, s
   }
 }
 
+size_t forcing_len(const nsb_ctx* c) { return (size_t)c->S.nc * (c->dim == 2 ? Fe<2>::NQ : Fe<3>::NQ) * c->dim; }
+
+// Both forcing slots are allocated (zeroed) together, the first time one of them receives values.
+void forcing_alloc(nsb_ctx* c) {
+  if (c->forcing[0].p) return;
+  for (auto& b : c->forcing) { b.alloc(forcing_len(c)); b.zero(c->stream); }
+}
+
+// Slot `which` now holds non-zero values or not.  A slot that is not set holds zeros while the other one is set (`written`:
+// its values were just overwritten, so they are zeroed even if it was clear before); both clear = both freed, and the
+// kernels read nothing.
+void forcing_commit(nsb_ctx* c, int which, bool nonzero, bool written) {
+  if (!nonzero && c->forcing_set[1 - which] && (written || c->forcing_set[which])) c->forcing[which].zero(c->stream);
+  c->forcing_set[which] = nonzero;
+  if (!c->forcing_set[0] && !c->forcing_set[1] && c->forcing[0].p) {
+    CK(cudaStreamSynchronize(c->stream));       // an assembly may still read them
+    for (auto& b : c->forcing) b.alloc(0);
+  }
+}
+
+// The vertices of the local cells (owned + ghost layer) and the local cell -> vertex table the evaluation kernel reads.
+void forcing_geometry(nsb_ctx* c) {
+  if (c->fsrc_geom) return;
+  const Structure& S = c->S;
+  const int dim = c->dim, NV = dim + 1;
+  std::vector<int> g2l(c->n_vertices, -1), cells((size_t)S.nc * NV);
+  std::vector<double> X;
+  for (int cl = 0; cl < S.nc; ++cl)
+    for (int v = 0; v < NV; ++v) {
+      const uint32_t g = c->cell_vertices[(size_t)S.cell_gid[cl] * NV + v];
+      if (g2l[g] < 0) {
+        g2l[g] = (int)(X.size() / dim);
+        X.insert(X.end(), c->coords.begin() + (size_t)g * dim, c->coords.begin() + (size_t)(g + 1) * dim);
+      }
+      cells[(size_t)cl * NV + v] = g2l[g];
+    }
+  c->fsrc_coords.upload(X, c->stream);
+  c->fsrc_cells.upload(cells, c->stream);
+  CK(cudaStreamSynchronize(c->stream));
+  c->fsrc_geom = true;
+}
+
+void forcing_unload(nsb_ctx* c) {
+  if (c->fsrc_lib) {
+    CK(cudaStreamSynchronize(c->stream));       // an evaluation may still run
+    CK(cudaLibraryUnload(c->fsrc_lib));
+  }
+  c->fsrc_lib = nullptr;
+  c->fsrc_kernel = nullptr;
+  c->fsrc_text.clear();
+}
+
 }  // namespace
 
 // =====================================================================================
@@ -1756,6 +1913,7 @@ int nsb_destroy(nsb_handle c) {
     try { close_peer_halo(c); nccl_barrier(c); } catch (...) {}
   }
   if (c->pin) cudaFreeHost(c->pin);
+  if (c->fsrc_lib) cudaLibraryUnload(c->fsrc_lib);
   if (c->comm) g_nccl.CommDestroy(c->comm);
   if (c->t0) cudaEventDestroy(c->t0);
   if (c->t1) cudaEventDestroy(c->t1);
@@ -1805,6 +1963,8 @@ int nsb_upload_mesh(nsb_handle c, int64_t n_vertices, const double* coords, int6
   CK(cudaSetDevice(c->device));
   for (auto& b : c->forcing) b.alloc(0);    // forcing values belong to the previous mesh's local cells
   c->forcing_set[0] = c->forcing_set[1] = false;
+  c->fsrc_coords.alloc(0); c->fsrc_cells.alloc(0);   // so does the geometry of a forcing source (the source itself stays)
+  c->fsrc_geom = false;
   const int dim = c->dim, NV = dim + 1;
   std::string e = build_structure(dim, n_vertices, coords, n_cells, cell_vertices, cell_dofs, n_u, n_p,
                                   c->nranks > 1 ? cell_part : nullptr, c->rank, c->nranks, c->S);
@@ -2089,26 +2249,135 @@ int nsb_set_forcing(nsb_handle c, int which, const double* f) {
     return fail(c, "nsb_set_forcing: which must be NSB_FORCING_NEW (0) or NSB_FORCING_OLD (1)");
   NSB_TRY
   CK(cudaSetDevice(c->device));
-  const size_t n = (size_t)c->S.nc * (c->dim == 2 ? Fe<2>::NQ : Fe<3>::NQ) * c->dim;
+  const size_t n = forcing_len(c);
   bool nonzero = false;
   if (f)
     for (size_t i = 0; i < n && !nonzero; ++i) nonzero = f[i] != 0.0;
   if (nonzero) {
-    if (!c->forcing[0].p) {
-      for (auto& b : c->forcing) { b.alloc(n); b.zero(c->stream); }
-    }
+    forcing_alloc(c);
     CK(cudaMemcpyAsync(c->forcing[which].p, f, n * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     CK(cudaStreamSynchronize(c->stream));       // f is the caller's pageable buffer
-  } else if (c->forcing_set[which] && c->forcing_set[1 - which]) {
-    c->forcing[which].zero(c->stream);
   }
-  c->forcing_set[which] = nonzero;
-  if (!c->forcing_set[0] && !c->forcing_set[1] && c->forcing[0].p) {
-    CK(cudaStreamSynchronize(c->stream));       // an assembly may still read them
-    for (auto& b : c->forcing) b.alloc(0);
-  }
+  forcing_commit(c, which, nonzero, false);
   return 0;
   NSB_CATCH(c)
+}
+
+int nsb_set_forcing_source(nsb_handle c, const char* src, const double* prm, int n_prm) {
+  if (!c || !c->have_mesh) return fail(c, "nsb_set_forcing_source: no mesh uploaded");
+  if (n_prm < 0 || n_prm > kForcingMaxParams)
+    return fail(c, "nsb_set_forcing_source: n_prm must be in 0.." + std::to_string(kForcingMaxParams) + ", got " + std::to_string(n_prm));
+  if (!prm && n_prm > 0) return fail(c, "nsb_set_forcing_source: prm is NULL but n_prm > 0");
+  NSB_TRY
+  CK(cudaSetDevice(c->device));
+  if (!src) {
+    forcing_unload(c);
+    forcing_commit(c, NSB_FORCING_NEW, false, false);
+    forcing_commit(c, NSB_FORCING_OLD, false, false);
+    c->fsrc_coords.alloc(0); c->fsrc_cells.alloc(0);
+    c->fsrc_geom = false;
+    return 0;
+  }
+  if (!c->fsrc_lib || c->fsrc_text != src) {
+    cudaDeviceProp prop;
+    CK(cudaGetDeviceProperties(&prop, c->device));
+    std::vector<char> cubin;
+    const std::string e = compile_forcing(c->dim, src, "sm_" + std::to_string(prop.major) + std::to_string(prop.minor) + "a", cubin);
+    if (!e.empty()) return fail(c, e);
+    forcing_unload(c);
+    CK(cudaLibraryLoadData(&c->fsrc_lib, cubin.data(), nullptr, nullptr, 0, nullptr, nullptr, 0));
+    CK(cudaLibraryGetKernel(&c->fsrc_kernel, c->fsrc_lib, "nsb_forcing_eval"));
+    c->fsrc_text = src;
+    ++c->fsrc_compiles;
+  }
+  std::vector<double> p(kForcingMaxParams, 0.0);
+  std::copy(prm, prm + n_prm, p.begin());
+  c->fsrc_prm.upload(p, c->stream);
+  if (!c->fsrc_flag.p) c->fsrc_flag.alloc(1);
+  forcing_geometry(c);                          // synchronises: p may go out of scope
+  return 0;
+  NSB_CATCH(c)
+}
+
+int nsb_eval_forcing(nsb_handle c, int which, double t) {
+  if (!c || !c->have_mesh) return fail(c, "nsb_eval_forcing: no mesh uploaded");
+  if (which != NSB_FORCING_NEW && which != NSB_FORCING_OLD)
+    return fail(c, "nsb_eval_forcing: which must be NSB_FORCING_NEW (0) or NSB_FORCING_OLD (1)");
+  if (!c->fsrc_lib) return fail(c, "nsb_eval_forcing: no forcing source set (nsb_set_forcing_source)");
+  NSB_TRY
+  CK(cudaSetDevice(c->device));
+  forcing_geometry(c);
+  forcing_alloc(c);
+  const int dim = c->dim, nq = dim == 2 ? Fe<2>::NQ : Fe<3>::NQ;
+  FeTables T;
+  fill_tables(dim, T);
+  double lam[Fe<3>::NQ * 4];                    // passed by value: [nq][dim + 1], the kernel's nsb_lambda
+  for (int q = 0; q < nq; ++q)
+    for (int v = 0; v <= dim; ++v) lam[q * (dim + 1) + v] = T.lam[q][v];
+  long long n_points = (long long)c->S.nc * nq;
+  const double* coords = c->fsrc_coords.p;
+  const int* cells = c->fsrc_cells.p;
+  const double* prm = c->fsrc_prm.p;
+  double* f = c->forcing[which].p;
+  unsigned int* flag = c->fsrc_flag.p;
+  void* args[] = {&coords, &cells, lam, &n_points, &t, &prm, &f, &flag};
+  CK(cudaMemsetAsync(flag, 0, sizeof(unsigned int), c->stream));
+  if (n_points > 0) {
+    const size_t id = c->prof.begin(PC_FORCING, c->stream);
+    CK(cudaLaunchKernel((const void*)c->fsrc_kernel, dim3(nblk(n_points, kForcingBlock)), dim3(kForcingBlock), args, 0, c->stream));
+    c->launch_check();
+    c->prof.end(id, c->stream);
+  }
+  unsigned int nonzero = 0;
+  CK(cudaMemcpyAsync(&nonzero, flag, sizeof(unsigned int), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  ++c->fsrc_evals;
+  forcing_commit(c, which, nonzero != 0, true);
+  return 0;
+  NSB_CATCH(c)
+}
+
+int nsb_get_forcing(nsb_handle c, int which, double* f) {
+  if (!c || !c->have_mesh) return fail(c, "nsb_get_forcing: no mesh uploaded");
+  if (which != NSB_FORCING_NEW && which != NSB_FORCING_OLD)
+    return fail(c, "nsb_get_forcing: which must be NSB_FORCING_NEW (0) or NSB_FORCING_OLD (1)");
+  if (!f) return fail(c, "nsb_get_forcing: f is NULL");
+  NSB_TRY
+  CK(cudaSetDevice(c->device));
+  const size_t n = forcing_len(c);
+  if (!c->forcing_set[which]) {
+    std::fill(f, f + n, 0.0);
+    return 1;
+  }
+  CK(cudaMemcpyAsync(f, c->forcing[which].p, n * sizeof(double), cudaMemcpyDeviceToHost, c->stream));
+  CK(cudaStreamSynchronize(c->stream));
+  return 0;
+  NSB_CATCH(c)
+}
+
+int nsb_forcing_info(nsb_handle c, int* has_source, int64_t* compiles, int64_t* evaluations, int* nvrtc_major, int* nvrtc_minor) {
+  if (!c) return -1;
+  g_nvrtc.load();
+  if (has_source) *has_source = c->fsrc_lib != nullptr;
+  if (compiles) *compiles = c->fsrc_compiles;
+  if (evaluations) *evaluations = c->fsrc_evals;
+  if (nvrtc_major) *nvrtc_major = g_nvrtc.major;
+  if (nvrtc_minor) *nvrtc_minor = g_nvrtc.minor;
+  return 0;
+}
+
+int nsb_check_forcing_source(int dim, const char* src, char* log, size_t log_size) {
+  std::string e;
+  std::vector<char> cubin;
+  if (dim != 2 && dim != 3) e = "nsb_check_forcing_source: dim must be 2 or 3";
+  else if (!src) e = "nsb_check_forcing_source: src is NULL";
+  else e = compile_forcing(dim, src, "sm_100a", cubin);
+  if (log && log_size) {
+    const size_t n = std::min(e.size(), log_size - 1);
+    std::memcpy(log, e.data(), n);
+    log[n] = '\0';
+  }
+  return e.empty() ? 0 : -1;
 }
 
 int nsb_get_vector(nsb_handle c, int which, double* vg) {

@@ -180,6 +180,17 @@ int nsh_set_forcing(nsh_handle h, nsh_forcing_fn fn, void* user) {
   NSH_CATCH
 }
 
+int nsh_set_forcing_source(nsh_handle h, const char* src, const double* prm, int32_t n_prm) {
+  if (!h) { g_err = "null handle"; return -1; }
+  NSH_TRY
+  if (n_prm < 0 || (n_prm > 0 && !prm)) { g_err = "nsh_set_forcing_source: bad parameter array"; return -1; }
+  const std::vector<double> p(prm, prm + n_prm);
+  if (h->dim == 2) h->s2->set_forcing_term(src ? std::make_shared<DeviceForcing<2>>(src, p) : nullptr);
+  else h->s3->set_forcing_term(src ? std::make_shared<DeviceForcing<3>>(src, p) : nullptr);
+  return 0;
+  NSH_CATCH
+}
+
 nsb_handle nsh_device(nsh_handle h) { return h->dim == 2 ? h->s2->device() : h->s3->device(); }
 
 // ---- host-only

@@ -139,6 +139,7 @@ template <int dim> void NavierStokes<dim>::setup() {
   forcing_points.clear();                                      // a new mesh has new local cells (and no forcing yet)
   forcing_time[0] = forcing_time[1] = std::nan("");
   forcing_on_device = false;
+  forcing_source_term = nullptr;
   pcout << "Setup complete." << std::endl;
 }
 
@@ -147,8 +148,32 @@ template <int dim> void NavierStokes<dim>::setup() {
 // so a halved retry samples t - dt/2 (cpp:688-697, 367-370; DESIGN.md section 1).  The default ForcingTerm and
 // Functions::ZeroFunction are identically zero: nothing is uploaded and the kernels read nothing.  The type test is exact
 // (typeid, not dynamic_cast), so a user class derived from ForcingTerm is evaluated.  A slot is re-evaluated only when its
-// time changes: the Newton iterations of one step reuse the upload.
+// time changes: the Newton iterations of one step reuse the upload.  A DeviceForcing is evaluated on the device instead: its
+// source is handed to the library once per term, and each slot whose time changed is filled by nsb_eval_forcing.
 template <int dim> void NavierStokes<dim>::update_forcing() {
+  if (const auto* df = dynamic_cast<const DeviceForcing<dim>*>(forcing_term.get())) {
+    if (forcing_source_term != forcing_term) {
+      ck(nsb_set_forcing_source(dev, df->source().c_str(), df->params().data(), (int)df->params().size()), "nsb_set_forcing_source");
+      forcing_source_term = forcing_term;
+    }
+    const double t_slot[2] = {time, time - deltat};            // NSB_FORCING_NEW, NSB_FORCING_OLD
+    const auto t0 = std::chrono::steady_clock::now();
+    for (int s = 0; s < 2; ++s) {
+      if (forcing_time[s] == t_slot[s]) continue;
+      forcing_time[s] = std::nan("");
+      ck(nsb_eval_forcing(dev, s, t_slot[s]), "nsb_eval_forcing");   // synchronises
+      forcing_time[s] = t_slot[s];
+      forcing_on_device = true;
+    }
+    step_forcing_seconds += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+    return;
+  }
+  if (forcing_source_term) {                                   // the term is no longer a DeviceForcing
+    ck(nsb_set_forcing_source(dev, nullptr, nullptr, 0), "nsb_set_forcing_source");
+    forcing_source_term = nullptr;
+    forcing_on_device = false;
+    forcing_time[0] = forcing_time[1] = std::nan("");
+  }
   const std::type_info& ft = typeid(*forcing_term);
   if (ft == typeid(ForcingTerm<dim>) || ft == typeid(Functions::ZeroFunction<dim>)) {
     if (forcing_on_device) {

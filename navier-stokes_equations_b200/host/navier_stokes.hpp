@@ -9,6 +9,7 @@
 #include <fstream>
 #include <iostream>
 #include <memory>
+#include <stdexcept>
 #include <string>
 #include <vector>
 
@@ -51,6 +52,24 @@ template <int dim> class ForcingTerm : public Function<dim> {
 public:
   ForcingTerm() : Function<dim>(dim + 1) {}
 };
+// A forcing term given as CUDA source (include/nsb200.h, nsb_set_forcing_source), evaluated on the device at the
+// quadrature points.  Immutable: to change the source or the parameters, call set_forcing_term with a new one.  There is
+// no host evaluation.
+template <int dim> class DeviceForcing : public Function<dim> {
+public:
+  explicit DeviceForcing(std::string source_, std::vector<double> params_ = {})
+    : Function<dim>(dim + 1), src(std::move(source_)), prm(std::move(params_)) {
+    if (prm.size() > 16) throw std::invalid_argument("DeviceForcing takes at most 16 parameters, got " + std::to_string(prm.size()));
+  }
+  double value(const Point<dim>& /*p*/, const unsigned int /*component*/ = 0) const override {
+    throw std::logic_error("DeviceForcing is evaluated on the GPU only (nsb_eval_forcing)");
+  }
+  const std::string& source() const { return src; }
+  const std::vector<double>& params() const { return prm; }
+private:
+  const std::string src;
+  const std::vector<double> prm;
+};
 template <int dim> class InitialCondition : public Function<dim> {
 public:
   InitialCondition() : Function<dim>(dim + 1) {}
@@ -87,7 +106,8 @@ struct StepInfo {
   double time = 0, cd = 0, cl = 0, dp = 0, wall_seconds = 0;
   int gmres_iterations = 0, newton_iterations = 0, solves = 0;
   bool converged = true;
-  double forcing_seconds = 0;     // host time spent evaluating and uploading the forcing term (part of wall_seconds)
+  double forcing_seconds = 0;     // time spent evaluating the forcing term and getting it to the device: host evaluation and
+                                  // upload, or device evaluation and its synchronise for a DeviceForcing (part of wall_seconds)
 };
 
 template <int dim> class NavierStokes {
@@ -201,6 +221,7 @@ protected:
   bool forcing_on_device = false;
   std::vector<Point<dim>> forcing_points;      // quadrature points of the device's local cells (nsb_get_quadrature_points)
   std::vector<Vector<double>> forcing_values;  // vector_value_list output, kept between evaluations
+  std::shared_ptr<Function<dim>> forcing_source_term;   // the DeviceForcing whose source the device holds, if any
 
   void push_params(bool first_order);
   void update_forcing();

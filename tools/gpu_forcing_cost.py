@@ -6,10 +6,15 @@
    its own repeats.
 2. The host side of one slot through the C ABI: exporting the quadrature points, evaluating a simple analytic forcing with
    numpy and uploading it (nsb_set_forcing).
-3. The host class (NavierStokes<3> through HostSolver.set_forcing): the per-step time of evaluating and uploading the
-   forcing that the step reports (StepInfo::forcing_seconds), next to the step's wall time.
+3. The same forcing as CUDA source evaluated on the device (nsb_set_forcing_source): NVRTC compile time without a GPU
+   (nsb_check_forcing_source) and the first set (compile, load, geometry upload); the `forcing` kernel's time per slot
+   from CUDA events, and the bytes it writes per second as a share of a device-to-device copy's bandwidth measured in the
+   same run (torch copy of 2 x 2 GB buffers, larger than L2: read + write bytes over time).
+4. The host class (NavierStokes<3> through HostSolver): unforced, with the Python callback (HostSolver.set_forcing) and
+   with the source (set_forcing_source): the per-step time the step reports for the forcing (StepInfo::forcing_seconds),
+   next to the step's wall time.
 The card's name and power limit are read in the same run.
-  python tools/gpu_forcing_cost.py [--level 20] [--rounds 5] [--launches 5] [--steps 2] [--json out.json]"""
+  python tools/gpu_forcing_cost.py [--level 20] [--rounds 5] [--launches 5] [--steps 2] [--evals 20] [--json out.json]"""
 import argparse
 import json
 import os
@@ -32,6 +37,31 @@ def analytic_forcing(x, t):
     return f
 
 
+# analytic_forcing as CUDA source (M_PI is not defined in NVRTC's built-ins)
+ANALYTIC_SRC = r"""
+__device__ void nsb_forcing(const double* x, double t, const double* prm, double* f) {
+  const double pi = 3.141592653589793;
+  f[2] = (1.0 + 0.5 * sin(t)) * sin(pi * x[0] / 0.41) * sin(pi * x[1] / 0.41);
+}
+"""
+
+
+def copy_bandwidth(nbytes=2 << 30, reps=10):
+    """Device-to-device copy: (read + write bytes) / time, CUDA events, buffers much larger than L2."""
+    import torch
+    a = torch.empty(nbytes, dtype=torch.uint8, device="cuda")
+    b = torch.empty_like(a)
+    for _ in range(2):
+        b.copy_(a)
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record()
+    for _ in range(reps):
+        b.copy_(a)
+    e1.record()
+    e1.synchronize()
+    return 2.0 * nbytes * reps / (e0.elapsed_time(e1) * 1e-3)
+
+
 def card():
     q = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
                        capture_output=True, text=True)
@@ -44,6 +74,7 @@ def main():
     ap.add_argument("--rounds", type=int, default=5)
     ap.add_argument("--launches", type=int, default=5)
     ap.add_argument("--steps", type=int, default=2)
+    ap.add_argument("--evals", type=int, default=20, help="timed nsb_eval_forcing calls per slot")
     ap.add_argument("--json", default=None)
     args = ap.parse_args()
     nsb = load_nsb()
@@ -114,18 +145,48 @@ def main():
     out["forcing_bytes_per_assembly"] = int(extra)
     print("asm_context per launch [ms]:", json.dumps(out["asm_context_ms"]), flush=True)
     print("extra bytes read per assembly: %.2f GB" % (extra / 1e9), flush=True)
+
+    # ---- the same forcing evaluated on the device from CUDA source
+    t0 = time.perf_counter()
+    nsb.check_forcing_source(3, ANALYTIC_SRC)
+    t1 = time.perf_counter()
+    dev.set_forcing_source(ANALYTIC_SRC)
+    t2 = time.perf_counter()
+    for which, t in ((nsb.NSB_FORCING_NEW, 1.0), (nsb.NSB_FORCING_OLD, 0.99)):       # warm
+        dev.eval_forcing(which, t)
+    fd = dev.forcing(nsb.NSB_FORCING_NEW)
+    dev_err = float(np.abs(fd - f_new).max() / np.abs(f_new).max())
+    dev.profile_enable(True)
+    dev.profile_reset()
+    t3 = time.perf_counter()
+    for k in range(args.evals):
+        dev.eval_forcing(k % 2, 1.0 - 0.01 * (k % 2))
+    t4 = time.perf_counter()
+    ms, n = dev.profile()["forcing"]
+    dev.profile_enable(False)
+    bw = copy_bandwidth()
+    kernel_ms = ms / n
+    written = int(f_new.nbytes)
+    out["device_source"] = dict(nvrtc=dev.forcing_info()["nvrtc"], compile_only_s=t1 - t0, first_set_s=t2 - t1,
+                                kernel_ms_per_slot=kernel_ms, eval_call_s_per_slot=(t4 - t3) / args.evals,
+                                bytes_written_per_slot=written, write_rate_GBps=written / (kernel_ms * 1e-3) / 1e9,
+                                copy_bandwidth_GBps=bw / 1e9, share_of_copy_bandwidth=written / (kernel_ms * 1e-3) / bw,
+                                max_rel_err_vs_numpy=dev_err)
+    print("device source:", json.dumps(out["device_source"]), flush=True)
+    dev.set_forcing_source(None)
     dev.close()
 
     # ---- the host class: evaluation + upload per step
     steps = {}
-    for forced in (False, True):
+    for mode in ("none", "callback", "source"):
         s = nsb.HostSolver("3D-2Z", mesh_file)
-        if forced:
+        if mode == "callback":
             s.set_forcing(analytic_forcing)
+        elif mode == "source":
+            s.set_forcing_source(ANALYTIC_SRC)
         s.initialize()
         infos = [s.step() for _ in range(args.steps)]
-        steps["forced" if forced else "none"] = [dict(wall_s=i["wall_seconds"], forcing_s=i["forcing_seconds"],
-                                                      gmres=i["gmres_iterations"]) for i in infos]
+        steps[mode] = [dict(wall_s=i["wall_seconds"], forcing_s=i["forcing_seconds"], gmres=i["gmres_iterations"]) for i in infos]
         s.close()
     out["host_class_steps"] = steps
     print("host class steps:", json.dumps(steps), flush=True)

@@ -4,8 +4,10 @@ the tight-tolerance solve against a sparse direct solve, the iteration count at 
 (partition-independent preconditioner), and three time steps of the C++ host class NavierStokes<3>(make_3D_2Z)
 (BASELINE config 3, "1 vs 2 GPUs") with per-rank VTU pieces.  --forcing adds a body force everywhere: each rank
 samples it at its own local cells' quadrature points (owned + ghost layer), the oracle at its own, and the host class
-takes it through HostSolver.set_forcing.
-  python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/gpu_multi.py [--json out.json] [--forcing]
+takes it through HostSolver.set_forcing.  --forcing-source does the same with the force given as CUDA source: every rank
+compiles it and evaluates it on the device at its own local cells (ghost layer included), and the slots are compared bit
+for bit with the single-GPU ones, cell by cell.
+  python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/gpu_multi.py [--json out.json] [--forcing | --forcing-source]
 tests/test_gpu_multirank.py and tests/test_gpu_forcing.py run this under pytest and assert on the JSON."""
 import argparse
 import json
@@ -25,6 +27,7 @@ from oracle import assemble as asm, dofs as odofs, postprocess as pp, solve as o
 import nsb200 as nsb  # noqa: E402
 from tests.conftest import synthetic_state  # noqa: E402
 from tests.forcing_cases import ForcedOracle, quadrature_points, sample, smooth_forcing  # noqa: E402
+from tests.forcing_sources import SMOOTH  # noqa: E402
 from tools import meshgen, msh  # noqa: E402
 
 
@@ -34,6 +37,7 @@ def main():
     ap.add_argument("--lc", type=float, default=0.04)
     ap.add_argument("--part", default="chunks", help="cell partition: chunks (contiguous) or metis (face-dual graph, like the reference)")
     ap.add_argument("--forcing", action="store_true", help="assemble and step with a non-zero body force")
+    ap.add_argument("--forcing-source", action="store_true", help="the same body force as CUDA source evaluated on each GPU")
     args = ap.parse_args()
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
@@ -49,8 +53,9 @@ def main():
     un, unm1 = synthetic_state(dm, 3, tc["U_m"])
     p = asm.Params(dt=0.01, theta=0.5, nu=1e-3, use_supg=True)
     t_new, t_old = 1.0, 0.99
+    forced = args.forcing or args.forcing_source
     forcing = None
-    if args.forcing:
+    if forced:
         qp = quadrature_points(mesh)
         forcing = (sample(smooth_forcing, qp, t_new), sample(smooth_forcing, qp, t_old))
     ref = asm.assemble(mesh, dm, pat, p, con, "linearized", un, unm1, forcing=forcing) if rank == 0 else None
@@ -63,6 +68,10 @@ def main():
         if args.forcing:
             qd = dev.quadrature_points()
             dev.set_forcing(sample(smooth_forcing, qd, t_new), sample(smooth_forcing, qd, t_old))
+        elif args.forcing_source:
+            dev.set_forcing_source(SMOOTH)
+            dev.eval_forcing(nsb.NSB_FORCING_NEW, t_new)
+            dev.eval_forcing(nsb.NSB_FORCING_OLD, t_old)
         dev.set_constraints(con.dofs, con.val[con.dofs])
         dev.set_params(0.01, 0.5, 1e-3, 1.0, 0.1, True, False)
         dev.set_vector(nsb.NSB_SOLUTION_OLD, un)
@@ -75,6 +84,12 @@ def main():
     vals1 = one.matrix_values()
     rp1, _ = one.pattern()
     b1 = one.get_vector(nsb.NSB_RHS)
+    if args.forcing_source:
+        # the single-GPU slots, cells keyed by their quadrature points (bit-identical on every rank: same vertices, same
+        # operations), so that each rank's local cells can be matched to them
+        q1 = one.quadrature_points()
+        fn1, fo1 = one.forcing(nsb.NSB_FORCING_NEW), one.forcing(nsb.NSB_FORCING_OLD)
+        slots1 = {q1[k].tobytes(): k for k in range(q1.shape[0])}
     one.assemble_pressure_matrices()
     ok1, it1, _ = one.solve(200, 1e-2, 150)
     one.close()
@@ -105,6 +120,11 @@ def main():
     b = dev.get_vector(nsb.NSB_RHS)
     errb = np.abs(b - ref.b).max() / np.abs(ref.b).max()
     b_bitexact = bool(np.array_equal(b, b1))
+    slots_bitexact = None
+    if args.forcing_source:
+        qd, fnd, fod = dev.quadrature_points(), dev.forcing(nsb.NSB_FORCING_NEW), dev.forcing(nsb.NSB_FORCING_OLD)
+        idx = [slots1.get(qd[k].tobytes(), -1) for k in range(qd.shape[0])]
+        slots_bitexact = bool(min(idx) >= 0 and np.array_equal(fnd, fn1[idx]) and np.array_equal(fod, fo1[idx]))
     dev.assemble_pressure_matrices()
     ok, it, res = dev.solve(200, 1e-2, 150)
     ok2, it2, _ = dev.solve(3000, 1e-12, 150)
@@ -115,7 +135,7 @@ def main():
     rec = dict(rank=rank, world=world, rows=int(nrows), cells=int(nc), pattern_ok=bool(okpat), A_relerr=float(errA),
                A_bitexact_vs_1gpu=bool(bitexact), b_relerr=float(errb), b_bitexact_vs_1gpu=b_bitexact,
                gmres_ok=bool(ok), gmres_its=int(it), gmres_its_1gpu=int(it1), tight_ok=bool(ok2), tight_its=int(it2),
-               field_relerr_vs_direct=ferr, fused=os.environ.get("NSB200_FUSED_HALO", "0"), halo=os.environ.get("NSB200_HALO", "p2p"))
+               field_relerr_vs_direct=ferr, slots_bitexact_vs_1gpu=slots_bitexact, fused=os.environ.get("NSB200_FUSED_HALO", "0"), halo=os.environ.get("NSB200_HALO", "p2p"))
     print("[rank %d/%d] " % (rank, world) + json.dumps(rec), flush=True)
     dist.barrier()
     dev.close()
@@ -132,11 +152,13 @@ def main():
                         write_vtu=True, output_dir=outdir, partitioner=1 if args.part == "metis" else 0)
     if args.forcing:
         hs.set_forcing(smooth_forcing)
+    elif args.forcing_source:
+        hs.set_forcing_source(SMOOTH)
     hs.initialize()
     infos = [hs.step() for _ in range(3)]
     steps = []
     if rank == 0:
-        o = ForcedOracle(mesh, "3D-2Z", smooth_forcing, solver="direct") if args.forcing else osolve.Oracle(mesh, "3D-2Z", solver="direct")
+        o = ForcedOracle(mesh, "3D-2Z", smooth_forcing, solver="direct") if forced else osolve.Oracle(mesh, "3D-2Z", solver="direct")
         for k, info in enumerate(infos):
             ref_ = o.step()
             errs = {key: abs(info[key] - ref_[key]) / max(abs(ref_[key]), 1e-300) for key in ("cd", "cl", "dp")}
@@ -156,7 +178,7 @@ def main():
         for src in pieces:
             piece = ET.parse(outdir + src).getroot().find("UnstructuredGrid/Piece")
             ncell += int(piece.get("NumberOfCells"))
-        summary = dict(world=world, partition=args.part, forcing=bool(args.forcing), fused=os.environ.get("NSB200_FUSED_HALO", "0"), halo=os.environ.get("NSB200_HALO", "p2p"), mesh_cells=int(mesh.n_cells), n_dofs=int(N),
+        summary = dict(world=world, partition=args.part, forcing=bool(args.forcing), forcing_source=bool(args.forcing_source), fused=os.environ.get("NSB200_FUSED_HALO", "0"), halo=os.environ.get("NSB200_HALO", "p2p"), mesh_cells=int(mesh.n_cells), n_dofs=int(N),
                        ranks=recs, host_class_steps=steps, host_class_field_relerr=field, vtu_pieces=pieces, vtu_cells_total=ncell)
         print("[summary] " + json.dumps(summary), flush=True)
         if args.json:
