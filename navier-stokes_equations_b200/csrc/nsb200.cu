@@ -9,6 +9,8 @@
 #include <nvrtc.h>  // types only: the library is resolved at run time (see NvrtcApi)
 
 #include <algorithm>
+#include <cerrno>
+#include <climits>
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -421,6 +423,7 @@ struct nsb_ctx {
   std::vector<std::unique_ptr<HaloBuf>> halo;
   int n_tiles_int = 0, n_tiles_bnd = 0;   // SpMV tiles without / with ghost reads
   std::vector<int> h_tiles_int, h_tiles_bnd, h_tile_node_ptr;     // host copies (fused halo tables)
+  int vs_ctas = 0;                  // NSB200_VS_CTAS: at most this many CTAs per streamed-operator launch (0: one per SM)
   bool fused_halo = false;          // halo exchange fused into the streamed operator (peer-store halo only): NSB200_FUSED_HALO=1.
                                     // Off by default: measured 4-5 % slower than the separate push / wait kernels on 2 GPUs (profiles/README.md)
   double* pin = nullptr;           // pinned staging buffer for host <-> device vector traffic (n_tot doubles)
@@ -630,7 +633,7 @@ template <int DIM, typename VT, int MODE, bool HALO>
 void launch_vel_stream(nsb_ctx* c, const VsDev& D, int ntiles, const int* list, const double* x, double* y, const double* u, double* poly,
                        PolyCoef pc, const VsHalo& hx) {
   if (ntiles <= 0) return;
-  const int grid = std::min(ntiles, c->num_sms);
+  const int grid = std::min(std::min(ntiles, c->num_sms), c->vs_ctas > 0 ? c->vs_ctas : ntiles);
   k_vel_stream<DIM, VT, MODE, HALO><<<grid, VS_THREADS, VsLayout<DIM, VT>::SMEM_BYTES, c->stream>>>(
       D.tiles, ntiles, list, reinterpret_cast<const VT*>(D.vals), D.meta, D.uniq_xoff, x, y, u, poly, pc, hx);
   c->launch_check();
@@ -1874,6 +1877,16 @@ int nsb_create(int dim, int device, nsb_handle* out) {
   c->dim = dim; c->device = device;
   *out = c;
   NSB_TRY
+  // NSB200_VS_CTAS=n caps the grid of the streamed velocity operator at n CTAs, so that every CTA walks its ring of stages
+  // through many tiles; the result does not depend on it (a tile is reduced by one consumer group in a fixed order)
+  if (const char* cap = std::getenv("NSB200_VS_CTAS")) {
+    char* end = nullptr;
+    errno = 0;
+    const long v = std::strtol(cap, &end, 10);
+    if (end == cap || *end != '\0' || errno == ERANGE || v < 1 || v > INT_MAX)
+      throw CudaErr{std::string("NSB200_VS_CTAS must be a positive integer, got \"") + cap + "\""};
+    c->vs_ctas = (int)v;
+  }
   int ndev = 0;
   CK(cudaGetDeviceCount(&ndev));
   if (device < 0 || device >= ndev) throw CudaErr{"no such CUDA device (the product path has no CPU fallback)"};

@@ -90,6 +90,12 @@ __device__ __forceinline__ void cp_async_arrive_noinc(uint64_t* bar) {
   asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
+// what the producer reads of a tile's global header: the tile (HALO: through the list), its value / metadata chunk and its
+// unique neighbour list
+struct VsHead {
+  int t, NQ, nq_off, u0, nuq;
+};
+
 struct VsHalo;
 template <int DIM> __device__ __forceinline__ void vs_deliver(const VsHalo& hx, int node, int comp, double v);
 
@@ -154,15 +160,48 @@ k_vel_stream(const VsTile* __restrict__ tiles, int n_tiles, const int* __restric
 
   if (warp == 0) {
     // ------------------------------------------------------------------ producer
+    // Software-pipelined so that no global round trip sits between "stage free" and "stage refilling": the headers of this
+    // CTA's tiles are loaded a batch of 32 ahead (lane j holds tile b + j; HALO: with the list entry) and read by shuffle, and
+    // the neighbour offsets of tile it + 1 are loaded as soon as the copies of tile it are issued, so they land while the
+    // producer waits for the next stage.  Between the wait on a stage and its copies there is nothing but shuffles.
+    constexpr int PER_LANE = VS_MAX_UNIQ / 32;
+    const int k0 = (int)blockIdx.x, dk = (int)gridDim.x;          // the it-th tile of this CTA is list position k0 + it * dk
+    auto fetch = [&](int b, VsHead& h) {
+      const int it = b + lane;
+      h = VsHead{0, 0, 0, 0, 0};
+      if (it < my_tiles) {
+        h.t = HALO ? __ldg(tile_list + k0 + it * dk) : k0 + it * dk;
+        const VsTile* hd = tiles + h.t;
+        h.NQ = __ldg(&hd->NQ); h.nq_off = __ldg(&hd->nq_off); h.u0 = __ldg(&hd->u0); h.nuq = __ldg(&hd->nuq);
+      }
+    };
+    // offsets of the unique neighbour nodes of tile `it` (-1: none), lane + 32 q
+    auto offsets = [&](int it, int u0, int nuq, int (&xo)[PER_LANE]) {
+#pragma unroll
+      for (int q = 0; q < PER_LANE; ++q) {
+        const int i = lane + 32 * q;
+        xo[q] = it < my_tiles && i < nuq ? __ldg(uniq_xoff + u0 + i) : -1;
+      }
+    };
+    VsHead cur, nxt;                               // headers of tiles [b, b + 32) and [b + 32, b + 64)
+    fetch(0, cur);
+    fetch(32, nxt);
+    int xo[PER_LANE];
+    offsets(0, __shfl_sync(NSB_FULL, cur.u0, 0), __shfl_sync(NSB_FULL, cur.nuq, 0), xo);
     bool waited = false;
     for (int it = 0; it < my_tiles; ++it) {
       const int s = it % S;
       const uint32_t ph = (uint32_t)(it / S) & 1u;
+      if (it > 0 && (it & 31) == 0) {
+        cur = nxt;
+        fetch(it + 32, nxt);
+      }
+      const int t = __shfl_sync(NSB_FULL, cur.t, it & 31);
+      const int NQ = __shfl_sync(NSB_FULL, cur.NQ, it & 31), nq_off = __shfl_sync(NSB_FULL, cur.nq_off, it & 31);
       if (it >= S) mbar_wait(empty + s, ph ^ 1u);                       // consumers released the stage's previous tile
-      int t = (int)blockIdx.x + it * (int)gridDim.x;
       bool ghosts = false;                         // this tile reads ghost entries delivered by peer stores
       if (HALO) {
-        ghosts = t >= hx.n_int;
+        ghosts = k0 + it * dk >= hx.n_int;
         if (ghosts && !waited) {
           // first boundary tile of this CTA: the peers' deliveries of x must have landed
           if (hx.wait_seq && lane < hx.npeers) {
@@ -173,27 +212,17 @@ k_vel_stream(const VsTile* __restrict__ tiles, int n_tiles, const int* __restric
           __syncwarp();
           waited = true;
         }
-        t = __ldg(tile_list + t);
       }
-      const VsTile* hd = tiles + t;
-      const int NQ = __ldg(&hd->NQ), nq_off = __ldg(&hd->nq_off), u0 = __ldg(&hd->u0), nuq = __ldg(&hd->nuq);
       unsigned char* st = vs_smem + s * L::STAGE_BYTES;
       if (lane == 0) {
         const uint32_t vb = (uint32_t)(PL * 4 * NQ * (int)sizeof(VT)), mb = (uint32_t)(NQ * 16);
         mbar_expect_tx(full + s, vb + mb + (uint32_t)L::HDR_BYTES);
-        tma_bulk_g2s(st + L::OFF_HDR, hd, L::HDR_BYTES, full + s);
+        tma_bulk_g2s(st + L::OFF_HDR, tiles + t, L::HDR_BYTES, full + s);
         tma_bulk_g2s(st + L::OFF_VAL, vals + (long long)PL * 4 * nq_off, vb, full + s);
         tma_bulk_g2s(st + L::OFF_META, meta + (long long)4 * nq_off, mb, full + s);
       }
-      // x values of the tile's unique neighbour nodes: all index loads first (independent, one round trip), then the copies
+      // x values of the tile's unique neighbour nodes
       double* xs = reinterpret_cast<double*>(st + L::OFF_XS);
-      constexpr int PER_LANE = VS_MAX_UNIQ / 32;
-      int xo[PER_LANE];
-#pragma unroll
-      for (int q = 0; q < PER_LANE; ++q) {
-        const int i = lane + 32 * q;
-        xo[q] = i < nuq ? __ldg(uniq_xoff + u0 + i) : -1;
-      }
       if (HALO && ghosts) {
         // ghost entries were written by other GPUs during this kernel: read those through L2 (an L1 line that straddles the
         // owned / ghost boundary may be stale) and store them; owned entries go the asynchronous way as usual
@@ -231,6 +260,11 @@ k_vel_stream(const VsTile* __restrict__ tiles, int n_tiles, const int* __restric
         }
         cp_async_arrive_noinc(full + s);
       }
+      // offsets of tile it + 1, whose header is in this batch or the next one
+      const bool in_cur = (it & 31) != 31;
+      const int u0 = __shfl_sync(NSB_FULL, in_cur ? cur.u0 : nxt.u0, (it + 1) & 31);
+      const int nuq = __shfl_sync(NSB_FULL, in_cur ? cur.nuq : nxt.nuq, (it + 1) & 31);
+      offsets(it + 1, u0, nuq, xo);
     }
     return;
   }
