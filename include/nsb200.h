@@ -214,7 +214,7 @@ int nsb_solver_info(nsb_handle h, int* poly_degree, double* poly_probe_residual,
 int nsb_velocity_operator_info(nsb_handle h, int* precision, int64_t* value_bytes, int64_t* index_bytes, int64_t* tiles,
                                int64_t* blocks);
 /* how the ghost entries travel: halo_mode 0 = single GPU, 1 = NCCL send/recv, 2 = peer stores over NVLink (CUDA IPC; separate
- * push / wait kernels), 3 = peer stores fused into the streamed velocity operator; doubles this rank sends per velocity exchange */
+ * push / wait kernels); doubles this rank sends per velocity exchange */
 int nsb_comm_info(nsb_handle h, int* nranks, int* halo_mode, int64_t* halo_doubles_per_exchange);
 /* inspection (parity tests): the Galerkin coarse operator P^T F P of the two-level velocity cycle as block CSR over the owned
  * vertices -- global vertex id of every row, block row pointer, global vertex id of every block column, dim*dim values per

@@ -328,7 +328,7 @@ class Device:
         a, b = C.c_int(), C.c_int()
         d = C.c_int64()
         self._ck(lib().nsb_comm_info(self.h, C.byref(a), C.byref(b), C.byref(d)))
-        return dict(nranks=a.value, halo=("none", "nccl send/recv", "peer stores over NVLink (CUDA IPC)", "peer stores fused into the streamed operator")[b.value],
+        return dict(nranks=a.value, halo=("none", "nccl send/recv", "peer stores over NVLink (CUDA IPC)")[b.value],
                     halo_doubles_per_exchange=d.value)
 
     def velocity_pc_info(self):

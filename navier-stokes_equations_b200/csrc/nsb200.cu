@@ -292,13 +292,6 @@ struct PeerHalo {
   unsigned long long seq = 0;
   const double* last_vec = nullptr;
   int total_f_vel = 0, total_f_all = 0, total_c = 0;
-  // fused delivery inside the streamed operator (VsHalo): per owned node / vertex the peers' landing offsets, the tile lists
-  // [tiles without ghost reads | tiles with], and which vector currently has a delivery in flight
-  DBuf<int> send_ptr_f, send_ptr_c, list_f, list_c;
-  DBuf<int2> send_dst_f, send_dst_c;
-  int n_int_f = 0, n_int_c = 0;
-  const double* fresh_vec = nullptr;       // its ghosts are being delivered by the kernel that produced it ...
-  unsigned long long fresh_seq = 0;        // ... under this sequence number
 };
 
 // device view of one streamed operator (velstream.cuh)
@@ -336,7 +329,6 @@ struct Coarse {
   DBuf<long long> nbr_ptr, vedge_ptr;
   DBuf<int> nbr_vxoff, vedge_xoff, ends_xoff, send_xoff;
   DBuf<double> cvals, dinv, rc, z0, z1, zd, poly, pin, send_buf;
-  std::vector<int> h_tiles_int, h_tiles_bnd, h_tile_node_ptr;
   std::vector<int64_t> gid, h_nbr_ptr, h_nbr_gid;     // host copies: global vertex ids of the owned rows / of the neighbours
   bool built = false, valid = false;   // structures uploaded / operator matches the assembled system
 };
@@ -421,11 +413,7 @@ struct nsb_ctx {
   double Mp_lmax = 1.0;
   std::vector<std::unique_ptr<DevLevel>> amg;
   std::vector<std::unique_ptr<HaloBuf>> halo;
-  int n_tiles_int = 0, n_tiles_bnd = 0;   // SpMV tiles without / with ghost reads
-  std::vector<int> h_tiles_int, h_tiles_bnd, h_tile_node_ptr;     // host copies (fused halo tables)
   int vs_ctas = 0;                  // NSB200_VS_CTAS: at most this many CTAs per streamed-operator launch (0: one per SM)
-  bool fused_halo = false;          // halo exchange fused into the streamed operator (peer-store halo only): NSB200_FUSED_HALO=1.
-                                    // Off by default: measured 4-5 % slower than the separate push / wait kernels on 2 GPUs (profiles/README.md)
   double* pin = nullptr;           // pinned staging buffer for host <-> device vector traffic (n_tot doubles)
   DBuf<double> coarse_inv;
   int coarse_n = 0;
@@ -487,7 +475,7 @@ void peer_wait(nsb_ctx* c) {
 }
 
 void peer_exchange(nsb_ctx* c, const double* v, int nseg, const DBuf<int>& seg_ptr, const DBuf<int>& src, const DBuf<long long>& land,
-                   int total_entries, bool wait = true) {
+                   int total_entries) {
   PeerHalo& H = c->ph;
   const int np = (int)c->S.peer.size();
   if (np == 0) return;
@@ -500,13 +488,12 @@ void peer_exchange(nsb_ctx* c, const double* v, int nseg, const DBuf<int>& seg_p
     c->launch_check();
   }
   H.last_vec = v;
-  H.fresh_vec = nullptr;
   ++H.seq;
   const int grid = std::max(1, std::min(nblk(total_entries, 256), 64));
   k_halo_push<<<grid, 256, 0, c->stream>>>(nseg, np, seg_ptr.p, src.p, land.p, H.d_peer_arena.p, vec_off, v, H.d_peer_flags.p, c->rank,
                                             H.seq, H.counter.p);
   c->launch_check();
-  if (wait) peer_wait(c);
+  peer_wait(c);
 }
 
 void halo_exchange(nsb_ctx* c, double* v, bool with_pressure = true) {
@@ -621,33 +608,29 @@ template <int DIM> void set_smem_attr(int bytes) {
 
 template <int DIM, typename VT> void set_vs_attr() {
   const int bytes = VsLayout<DIM, VT>::SMEM_BYTES;
-  CK(cudaFuncSetAttribute(k_vel_stream<DIM, VT, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  CK(cudaFuncSetAttribute(k_vel_stream<DIM, VT, 3, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  CK(cudaFuncSetAttribute(k_vel_stream<DIM, VT, 3, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  CK(cudaFuncSetAttribute(k_vel_stream<DIM, VT, 4, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
-  CK(cudaFuncSetAttribute(k_vel_stream<DIM, VT, 4, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  CK(cudaFuncSetAttribute(k_vel_stream<DIM, VT, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  CK(cudaFuncSetAttribute(k_vel_stream<DIM, VT, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+  CK(cudaFuncSetAttribute(k_vel_stream<DIM, VT, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
 }
 
-// one application of the streamed operator over `ntiles` tiles (all of them, or the listed ones)
-template <int DIM, typename VT, int MODE, bool HALO>
-void launch_vel_stream(nsb_ctx* c, const VsDev& D, int ntiles, const int* list, const double* x, double* y, const double* u, double* poly,
-                       PolyCoef pc, const VsHalo& hx) {
-  if (ntiles <= 0) return;
-  const int grid = std::min(std::min(ntiles, c->num_sms), c->vs_ctas > 0 ? c->vs_ctas : ntiles);
-  k_vel_stream<DIM, VT, MODE, HALO><<<grid, VS_THREADS, VsLayout<DIM, VT>::SMEM_BYTES, c->stream>>>(
-      D.tiles, ntiles, list, reinterpret_cast<const VT*>(D.vals), D.meta, D.uniq_xoff, x, y, u, poly, pc, hx);
+// one application of the streamed operator over all tiles of D
+template <int DIM, typename VT, int MODE>
+void launch_vel_stream(nsb_ctx* c, const VsDev& D, const double* x, double* y, const double* u, double* poly, PolyCoef pc) {
+  if (D.n_tiles <= 0) return;
+  const int grid = std::min(std::min(D.n_tiles, c->num_sms), c->vs_ctas > 0 ? c->vs_ctas : D.n_tiles);
+  k_vel_stream<DIM, VT, MODE><<<grid, VS_THREADS, VsLayout<DIM, VT>::SMEM_BYTES, c->stream>>>(
+      D.tiles, reinterpret_cast<const VT*>(D.vals), D.meta, D.uniq_xoff, x, y, u, poly, pc, D.n_tiles);
   c->launch_check();
 }
-template <int MODE, bool HALO>
-void vel_stream(nsb_ctx* c, const VsDev& D, int ntiles, const int* list, const double* x, double* y, const double* u, double* poly, PolyCoef pc,
-                const VsHalo& hx = VsHalo{}) {
+template <int MODE>
+void vel_stream(nsb_ctx* c, const VsDev& D, const double* x, double* y, const double* u, double* poly, PolyCoef pc) {
   const bool h = c->opt.precond_precision == 16;
   if (c->dim == 2) {
-    if (h) launch_vel_stream<2, __half, MODE, HALO>(c, D, ntiles, list, x, y, u, poly, pc, hx);
-    else launch_vel_stream<2, float, MODE, HALO>(c, D, ntiles, list, x, y, u, poly, pc, hx);
+    if (h) launch_vel_stream<2, __half, MODE>(c, D, x, y, u, poly, pc);
+    else launch_vel_stream<2, float, MODE>(c, D, x, y, u, poly, pc);
   } else {
-    if (h) launch_vel_stream<3, __half, MODE, HALO>(c, D, ntiles, list, x, y, u, poly, pc, hx);
-    else launch_vel_stream<3, float, MODE, HALO>(c, D, ntiles, list, x, y, u, poly, pc, hx);
+    if (h) launch_vel_stream<3, __half, MODE>(c, D, x, y, u, poly, pc);
+    else launch_vel_stream<3, float, MODE>(c, D, x, y, u, poly, pc);
   }
 }
 VsDev fine_dev(const nsb_ctx* c);
@@ -666,57 +649,13 @@ void spmv_vel(nsb_ctx* c, const double* x, double* y, const double* u, double* p
   size_t id = c->prof.begin(PC_SPMV_VEL, c->stream);
   const int g = c->n_stiles;
   if (c->vs_valid && MODE != 0) {
-    vel_stream<MODE == 0 ? 2 : MODE, false>(c, fine_dev(c), g, nullptr, x, y, u, poly, pc);
+    vel_stream<MODE == 0 ? 2 : MODE>(c, fine_dev(c), x, y, u, poly, pc);
   } else {
     if (c->dim == 2) k_spmv_vel<2, MODE, double><<<g, SPMV_WARPS * 32, 0, c->stream>>>(c->M, c->stiles, c->vals.p, x, y, u, poly, c->dinv.p, pc);
     else k_spmv_vel<3, MODE, double><<<g, SPMV_WARPS * 32, 0, c->stream>>>(c->M, c->stiles, c->vals.p, x, y, u, poly, c->dinv.p, pc);
     c->launch_check();
   }
   c->prof.end(id, c->stream);
-}
-
-// Operator application with the halo exchange fused into the streamed kernel (VsHalo, velstream.cuh): x's ghosts are either
-// already being delivered by the kernel that produced x (then this kernel waits for the peers' flags itself, behind its
-// interior tiles) or are exchanged by the separate push / wait kernels first; y's boundary rows are delivered to the peers
-// by this kernel.  MODE 3 or 4.
-template <int MODE>
-void fused_apply(nsb_ctx* c, bool coarse, const VsDev& D, double* x, double* y, const double* u, double* poly, PolyCoef pc) {
-  PeerHalo& H = c->ph;
-  const int np = (int)c->S.peer.size();
-  VsHalo hx{};
-  hx.flags = H.flags.p; hx.peer_rank = H.d_peer_rank.p; hx.npeers = np;
-  hx.n_int = coarse ? H.n_int_c : H.n_int_f;
-  hx.ghost_start = coarse ? c->dim * c->S.np_own : (int)c->S.n_own_dofs();
-  if (x == H.fresh_vec) hx.wait_seq = H.fresh_seq;
-  else {
-    if (coarse) peer_exchange(c, x, np, H.seg_ptr_c, H.src_c, H.land_c, H.total_c);
-    else peer_exchange(c, x, np, H.seg_ptr_f, H.src_f, H.land_f, H.total_f_vel);
-    hx.wait_seq = 0;
-  }
-  hx.send_ptr = coarse ? H.send_ptr_c.p : H.send_ptr_f.p;
-  hx.send_dst = coarse ? H.send_dst_c.p : H.send_dst_f.p;
-  hx.peer_arena = H.d_peer_arena.p;
-  hx.y_off = y - H.arena.p;
-  if (hx.y_off < 0 || (size_t)hx.y_off >= H.arena.n) throw CudaErr{"fused halo delivery into a vector outside the symmetric arena"};
-  hx.peer_flags = H.d_peer_flags.p; hx.my_rank = c->rank;
-  hx.push_seq = ++H.seq;
-  hx.counter = H.counter.p;
-  const int* list = coarse ? H.list_c.p : H.list_f.p;
-  vel_stream<MODE, true>(c, D, D.n_tiles, list, x, y, u, poly, pc, hx);
-  H.fresh_vec = y; H.fresh_seq = hx.push_seq;
-  H.last_vec = nullptr;
-}
-
-// one root of the velocity polynomial on a vector whose ghosts are stale
-void halo_spmv_vel3(nsb_ctx* c, double* x, double* y, const double* u, double* poly, PolyCoef pc) {
-  if (c->nranks > 1 && c->ph.on && c->vs_valid && c->fused_halo) {
-    size_t id = c->prof.begin(PC_SPMV_VEL, c->stream);
-    fused_apply<3>(c, false, fine_dev(c), x, y, u, poly, pc);
-    c->prof.end(id, c->stream);
-    return;
-  }
-  halo_exchange(c, x, false);
-  spmv_vel<3>(c, x, y, u, poly, pc);
 }
 
 void block_scale(nsb_ctx* c, const double* x, double* y) {
@@ -803,20 +742,13 @@ template <int MODE>
 void level_apply(nsb_ctx* c, PolyLevel& lv, const double* x, double* y, const double* u, double* poly, PolyCoef pc) {
   if (!lv.coarse) { spmv_vel<MODE>(c, x, y, u, poly, pc); return; }
   size_t id = c->prof.begin(PC_COARSE, c->stream);
-  vel_stream<MODE, false>(c, coarse_dev(c), c->cg.n_tiles, nullptr, x, y, u, poly, pc);
+  vel_stream<MODE>(c, coarse_dev(c), x, y, u, poly, pc);
   c->prof.end(id, c->stream);
 }
 
 // one root of a product-form polynomial on a vector whose ghosts are stale
 void level_root(nsb_ctx* c, PolyLevel& lv, double* x, double* y, const double* u, double* poly, PolyCoef pc) {
-  if (!lv.coarse) { halo_spmv_vel3(c, x, y, u, poly, pc); return; }
-  if (c->nranks > 1 && c->ph.on && c->fused_halo) {
-    size_t id = c->prof.begin(PC_COARSE, c->stream);
-    fused_apply<3>(c, true, coarse_dev(c), x, y, u, poly, pc);
-    c->prof.end(id, c->stream);
-    return;
-  }
-  halo_exchange_coarse(c, x);
+  level_halo(c, lv, x);
   level_apply<3>(c, lv, x, y, u, poly, pc);
 }
 
@@ -1102,14 +1034,8 @@ void apply_velocity_pc(nsb_ctx* c, const double* x) {
   c->prof.end(id, c->stream);
   // ---- smoothing from y0:  y = y0 + q(B) (Dinv x - B y0)
   level_block_scale(c, F, x, c->w_u.p);
-  if (c->nranks > 1 && c->ph.on && c->fused_halo) {
-    size_t idf = c->prof.begin(PC_SPMV_VEL, c->stream);
-    fused_apply<4>(c, false, fine_dev(c), y0, F.z0, c->w_u.p, nullptr, PolyCoef{1.0, -1.0, 0.0, 0.0});
-    c->prof.end(idf, c->stream);
-  } else {
-    halo_exchange(c, y0, false);
-    level_apply<4>(c, F, y0, F.z0, c->w_u.p, nullptr, PolyCoef{1.0, -1.0, 0.0, 0.0});
-  }
+  halo_exchange(c, y0, false);
+  level_apply<4>(c, F, y0, F.z0, c->w_u.p, nullptr, PolyCoef{1.0, -1.0, 0.0, 0.0});
   apply_poly(c, F);
   k_axpby<<<nblk(nu, 256), 256, 0, c->stream>>>(nu, 1.0, y0, 1.0, F.poly);
   c->launch_check();
@@ -1379,8 +1305,6 @@ void build_tiles(nsb_ctx* c) {
     if (!err2.empty()) throw CudaErr{err2};
     c->n_stiles = P.n_tiles();
     c->d_stile_ptr.upload(P.node_ptr, c->stream);
-    c->n_tiles_int = (int)P.tiles_int.size(); c->n_tiles_bnd = (int)P.tiles_bnd.size();
-    c->h_tiles_int = P.tiles_int; c->h_tiles_bnd = P.tiles_bnd; c->h_tile_node_ptr = P.node_ptr;
     c->d_suniq_ptr.upload(P.uniq_ptr, c->stream); c->d_suniq_xoff.upload(P.uniq_xoff, c->stream);
     c->d_spuniq_ptr.upload(P.puniq_ptr, c->stream); c->d_spuniq_xoff.upload(P.puniq_xoff, c->stream);
     c->d_nbr_loc.upload(P.nbr_loc, c->stream); c->d_pnbr_loc.upload(P.pnbr_loc, c->stream);
@@ -1529,39 +1453,6 @@ void setup_peer_halo(nsb_ctx* c, std::vector<DBuf<double>*> fine, std::vector<DB
   H.seg_ptr_f.upload(sp, st); H.src_f.upload(src, st); H.land_f.upload(land, st);
   H.seg_ptr_c.upload(spc, st); H.src_c.upload(srcc, st); H.land_c.upload(landc, st);
   H.d_peer_arena.upload(H.peer_arena, st); H.d_peer_flags.upload(H.peer_flags, st); H.d_peer_rank.upload(pr, st);
-  // fused delivery: per owned node (vertex) the landing offsets in the peers, and the tile lists interior-first
-  auto fused_tables = [&](int n_own, const std::vector<std::vector<int>>& send, const std::vector<long long>& landing, const std::vector<int>& /*t_int*/,
-                          const std::vector<int>& t_bnd, const std::vector<int>& node_ptr, DBuf<int>& d_ptr, DBuf<int2>& d_dst, DBuf<int>& d_list,
-                          int& n_int) {
-    std::vector<int> cnt(n_own + 1, 0);
-    for (int k = 0; k < np; ++k) for (int n : send[k]) cnt[n + 1]++;
-    for (int n = 0; n < n_own; ++n) cnt[n + 1] += cnt[n];
-    std::vector<int2> dst(cnt[n_own]);
-    std::vector<int> fill(cnt.begin(), cnt.end() - 1);
-    for (int k = 0; k < np; ++k)
-      for (size_t i = 0; i < send[k].size(); ++i) dst[fill[send[k][i]]++] = make_int2(k, (int)(landing[k] + (long long)i * dim));
-    // tiles that read ghosts or hold a sent node go to the back of the list: they run after the CTA has seen the peers'
-    // flags, which is also what makes delivering into the peers' buffers safe.  (A sent fine node always has a ghost
-    // neighbour; a sent VERTEX need not have a ghost vertex neighbour -- the peer may only own line nodes next to it.)
-    std::vector<char> back(node_ptr.size() - 1, 0);
-    for (int t : t_bnd) back[t] = 1;
-    for (size_t t = 0; t + 1 < node_ptr.size(); ++t)
-      for (int n = node_ptr[t]; n < node_ptr[t + 1] && !back[t]; ++n)
-        if (cnt[n + 1] != cnt[n]) back[t] = 1;
-    std::vector<int> list;
-    for (size_t t = 0; t + 1 < node_ptr.size(); ++t) if (!back[t]) list.push_back((int)t);
-    n_int = (int)list.size();
-    for (size_t t = 0; t + 1 < node_ptr.size(); ++t) if (back[t]) list.push_back((int)t);
-    for (auto& d : dst) if (d.y < 0) throw CudaErr{"halo plan: negative landing offset"};
-    d_ptr.upload(cnt, st); d_dst.upload(dst, st); d_list.upload(list, st);
-    CK(cudaStreamSynchronize(st));
-  };
-  {
-    std::vector<long long> lf(land.begin(), land.begin() + np);
-    fused_tables(S.nn_own, S.send_nodes, lf, c->h_tiles_int, c->h_tiles_bnd, c->h_tile_node_ptr, H.send_ptr_f, H.send_dst_f, H.list_f, H.n_int_f);
-    fused_tables(S.np_own, S.send_pids, landc, c->cg.h_tiles_int, c->cg.h_tiles_bnd, c->cg.h_tile_node_ptr, H.send_ptr_c, H.send_dst_c, H.list_c, H.n_int_c);
-  }
-  H.fresh_vec = nullptr; H.fresh_seq = 0;
   CK(cudaStreamSynchronize(st));
   nccl_barrier(c);                                   // every rank's flags are zeroed before anybody pushes
   H.on = true;
@@ -1590,7 +1481,6 @@ void build_coarse_level(nsb_ctx* c) {
   const int dim = c->dim;
   G.n_tiles = P.n_tiles();
   G.total_nq = V.total_nq;
-  G.h_tiles_int = P.tiles_int; G.h_tiles_bnd = P.tiles_bnd; G.h_tile_node_ptr = P.node_ptr;
   G.tiles.upload(V.tiles, st); G.meta.upload(V.meta, st); G.uniq_xoff.upload(P.uniq_xoff, st);
   std::vector<long long> t64(Sc.nbr_ptr.begin(), Sc.nbr_ptr.end()), v64(CL.vedge_ptr.begin(), CL.vedge_ptr.end());
   G.nbr_ptr.upload(t64, st); G.vedge_ptr.upload(v64, st);
@@ -1959,9 +1849,6 @@ int nsb_comm_init(nsb_handle c, int rank, int nranks, const void* uid) {
     ncclUniqueId id;
     std::memcpy(&id, uid, sizeof(id));
     CKN(g_nccl.CommInitRank(&c->comm, nranks, id, rank));
-    // NSB200_FUSED_HALO=1: halo exchange fused into the streamed velocity operator (peer-store halo only, DESIGN.md section 6)
-    const char* fh = std::getenv("NSB200_FUSED_HALO");
-    c->fused_halo = fh && fh[0] == '1';
   }
   c->rank = rank; c->nranks = nranks;
   return 0;
@@ -2931,7 +2818,7 @@ int nsb_velocity_operator_info(nsb_handle c, int* precision, int64_t* value_byte
 int nsb_comm_info(nsb_handle c, int* nranks, int* halo_mode, int64_t* halo_doubles_per_exchange) {
   if (!c) return -1;
   if (nranks) *nranks = c->nranks;
-  if (halo_mode) *halo_mode = c->nranks == 1 ? 0 : !c->ph.on ? 1 : c->fused_halo ? 3 : 2;
+  if (halo_mode) *halo_mode = c->nranks == 1 ? 0 : !c->ph.on ? 1 : 2;
   if (halo_doubles_per_exchange) {
     int64_t t = 0;
     for (size_t k = 0; k < c->S.peer.size(); ++k) t += (int64_t)c->S.send_nodes[k].size() * c->dim;

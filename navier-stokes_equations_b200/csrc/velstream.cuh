@@ -90,14 +90,10 @@ __device__ __forceinline__ void cp_async_arrive_noinc(uint64_t* bar) {
   asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 
-// what the producer reads of a tile's global header: the tile (HALO: through the list), its value / metadata chunk and its
-// unique neighbour list
+// what the producer reads of a tile's global header: the tile, its value / metadata chunk and its unique neighbour list
 struct VsHead {
   int t, NQ, nq_off, u0, nuq;
 };
-
-struct VsHalo;
-template <int DIM> __device__ __forceinline__ void vs_deliver(const VsHalo& hx, int node, int comp, double v);
 
 // the four values of one quad of one plane
 __device__ __forceinline__ void vs_load4(const float* p, double (&v)[4]) {
@@ -110,37 +106,13 @@ __device__ __forceinline__ void vs_load4(const __half* p, double (&v)[4]) {
   v[0] = (double)a.x; v[1] = (double)a.y; v[2] = (double)b.x; v[3] = (double)b.y;
 }
 
-// Halo exchange FUSED into the operator (several GPUs, peer-store halo of nsb200.cu): the kernel that produces y also
-// delivers it -- the epilogue of a boundary tile stores the rows other ranks hold as ghosts straight into the peers' copies
-// of y over NVLink, and the last consumer warp of the grid to finish raises this rank's sequence flag in every peer -- and
-// the kernel that consumes x waits for the peers' flags itself: tiles are taken from a list with the tiles that read no
-// ghost entry first, and a CTA's producer warp polls the flags only when it reaches its first boundary tile.  A chain of
-// polynomial roots is therefore ONE launch per root, with the exchange hidden behind the interior tiles.
-struct VsHalo {
-  // consuming x
-  const unsigned long long* flags;        // this rank's flag array (sequence numbers written by the peers)
-  const int* peer_rank;
-  int npeers;
-  int n_int;                              // tiles [0, n_int) of the list read no ghost entry
-  unsigned long long wait_seq;            // boundary tiles wait until every peer has reached it (0: ghosts already valid)
-  int ghost_start;                        // offsets >= this are ghost entries of x
-  // delivering y
-  const int* send_ptr;                    // [owned nodes + 1] -> send_dst
-  const int2* send_dst;                   // (peer index, offset of the node's first component inside the peer's vector)
-  double* const* peer_arena;
-  long long y_off;                        // offset of y inside the symmetric arena
-  unsigned long long* const* peer_flags;
-  int my_rank;
-  unsigned long long push_seq;
-  unsigned int* counter;                  // consumer warps of the grid that are done
-};
-
-// HALO: the k-th tile of this launch is tile_list[k], and the exchange of x / y is fused as described above.
-template <int DIM, typename VT, int MODE, bool HALO>
+// n_tiles comes last so that the pointer pairs and pc sit 16-byte aligned in the parameter bank: the epilogue then reads
+// them with 128-bit uniform loads
+template <int DIM, typename VT, int MODE>
 __global__ void __launch_bounds__(VS_THREADS, 1)
-k_vel_stream(const VsTile* __restrict__ tiles, int n_tiles, const int* __restrict__ tile_list, const VT* __restrict__ vals,
-             const uint32_t* __restrict__ meta, const int* __restrict__ uniq_xoff, const double* __restrict__ x,
-             double* __restrict__ y, const double* __restrict__ u, double* __restrict__ poly, PolyCoef pc, VsHalo hx) {
+k_vel_stream(const VsTile* __restrict__ tiles, const VT* __restrict__ vals, const uint32_t* __restrict__ meta,
+             const int* __restrict__ uniq_xoff, const double* __restrict__ x, double* __restrict__ y,
+             const double* __restrict__ u, double* __restrict__ poly, PolyCoef pc, int n_tiles) {
   using L = VsLayout<DIM, VT>;
   constexpr int PL = L::PL;
   constexpr int S = L::STAGES;
@@ -161,16 +133,16 @@ k_vel_stream(const VsTile* __restrict__ tiles, int n_tiles, const int* __restric
   if (warp == 0) {
     // ------------------------------------------------------------------ producer
     // Software-pipelined so that no global round trip sits between "stage free" and "stage refilling": the headers of this
-    // CTA's tiles are loaded a batch of 32 ahead (lane j holds tile b + j; HALO: with the list entry) and read by shuffle, and
-    // the neighbour offsets of tile it + 1 are loaded as soon as the copies of tile it are issued, so they land while the
-    // producer waits for the next stage.  Between the wait on a stage and its copies there is nothing but shuffles.
+    // CTA's tiles are loaded a batch of 32 ahead (lane j holds tile b + j) and read by shuffle, and the neighbour offsets of
+    // tile it + 1 are loaded as soon as the copies of tile it are issued, so they land while the producer waits for the next
+    // stage.  Between the wait on a stage and its copies there is nothing but shuffles.
     constexpr int PER_LANE = VS_MAX_UNIQ / 32;
-    const int k0 = (int)blockIdx.x, dk = (int)gridDim.x;          // the it-th tile of this CTA is list position k0 + it * dk
+    const int k0 = (int)blockIdx.x, dk = (int)gridDim.x;          // the it-th tile of this CTA is k0 + it * dk
     auto fetch = [&](int b, VsHead& h) {
       const int it = b + lane;
       h = VsHead{0, 0, 0, 0, 0};
       if (it < my_tiles) {
-        h.t = HALO ? __ldg(tile_list + k0 + it * dk) : k0 + it * dk;
+        h.t = k0 + it * dk;
         const VsTile* hd = tiles + h.t;
         h.NQ = __ldg(&hd->NQ); h.nq_off = __ldg(&hd->nq_off); h.u0 = __ldg(&hd->u0); h.nuq = __ldg(&hd->nuq);
       }
@@ -188,7 +160,6 @@ k_vel_stream(const VsTile* __restrict__ tiles, int n_tiles, const int* __restric
     fetch(32, nxt);
     int xo[PER_LANE];
     offsets(0, __shfl_sync(NSB_FULL, cur.u0, 0), __shfl_sync(NSB_FULL, cur.nuq, 0), xo);
-    bool waited = false;
     for (int it = 0; it < my_tiles; ++it) {
       const int s = it % S;
       const uint32_t ph = (uint32_t)(it / S) & 1u;
@@ -199,20 +170,6 @@ k_vel_stream(const VsTile* __restrict__ tiles, int n_tiles, const int* __restric
       const int t = __shfl_sync(NSB_FULL, cur.t, it & 31);
       const int NQ = __shfl_sync(NSB_FULL, cur.NQ, it & 31), nq_off = __shfl_sync(NSB_FULL, cur.nq_off, it & 31);
       if (it >= S) mbar_wait(empty + s, ph ^ 1u);                       // consumers released the stage's previous tile
-      bool ghosts = false;                         // this tile reads ghost entries delivered by peer stores
-      if (HALO) {
-        ghosts = k0 + it * dk >= hx.n_int;
-        if (ghosts && !waited) {
-          // first boundary tile of this CTA: the peers' deliveries of x must have landed
-          if (hx.wait_seq && lane < hx.npeers) {
-            const volatile unsigned long long* f = hx.flags + hx.peer_rank[lane];
-            while (*f < hx.wait_seq) { }
-          }
-          __threadfence_system();
-          __syncwarp();
-          waited = true;
-        }
-      }
       unsigned char* st = vs_smem + s * L::STAGE_BYTES;
       if (lane == 0) {
         const uint32_t vb = (uint32_t)(PL * 4 * NQ * (int)sizeof(VT)), mb = (uint32_t)(NQ * 16);
@@ -223,43 +180,15 @@ k_vel_stream(const VsTile* __restrict__ tiles, int n_tiles, const int* __restric
       }
       // x values of the tile's unique neighbour nodes
       double* xs = reinterpret_cast<double*>(st + L::OFF_XS);
-      if (HALO && ghosts) {
-        // ghost entries were written by other GPUs during this kernel: read those through L2 (an L1 line that straddles the
-        // owned / ghost boundary may be stale) and store them; owned entries go the asynchronous way as usual
 #pragma unroll
-        for (int q0 = 0; q0 < PER_LANE; q0 += 4) {
-          double gv[4][DIM];
+      for (int q = 0; q < PER_LANE; ++q) {
+        if (xo[q] >= 0) {
+          const int i = lane + 32 * q;
 #pragma unroll
-          for (int q = q0; q < q0 + 4; ++q)
-            if (xo[q] >= hx.ghost_start) {
-#pragma unroll
-              for (int c = 0; c < DIM; ++c) gv[q - q0][c] = __ldcg(x + xo[q] + c);
-            }
-#pragma unroll
-          for (int q = q0; q < q0 + 4; ++q) {
-            const int i = lane + 32 * q;
-            if (xo[q] >= hx.ghost_start) {
-#pragma unroll
-              for (int c = 0; c < DIM; ++c) xs[i * DIM + c] = gv[q - q0][c];
-            } else if (xo[q] >= 0) {
-#pragma unroll
-              for (int c = 0; c < DIM; ++c) cp_async_8(xs + i * DIM + c, x + xo[q] + c);
-            }
-          }
+          for (int c = 0; c < DIM; ++c) cp_async_8(xs + i * DIM + c, x + xo[q] + c);
         }
-        __threadfence_block();                     // the plain stores above precede the arrival
-        cp_async_arrive_noinc(full + s);
-      } else {
-#pragma unroll
-        for (int q = 0; q < PER_LANE; ++q) {
-          if (xo[q] >= 0) {
-            const int i = lane + 32 * q;
-#pragma unroll
-            for (int c = 0; c < DIM; ++c) cp_async_8(xs + i * DIM + c, x + xo[q] + c);
-          }
-        }
-        cp_async_arrive_noinc(full + s);
       }
+      cp_async_arrive_noinc(full + s);
       // offsets of tile it + 1, whose header is in this batch or the next one
       const bool in_cur = (it & 31) != 31;
       const int u0 = __shfl_sync(NSB_FULL, in_cur ? cur.u0 : nxt.u0, (it + 1) & 31);
@@ -367,48 +296,20 @@ k_vel_stream(const VsTile* __restrict__ tiles, int n_tiles, const int* __restric
     }
     __syncwarp();                                 // this warp's node sums are in ys
     // ---- fused epilogue over this warp's rows (contiguous in memory)
-    const bool deliver = HALO && hx.push_seq && ((int)blockIdx.x + it * (int)gridDim.x) >= hx.n_int;
     for (int i = r0 + lane, q = 0; i < r1; i += 32, ++q) {
       const double t = ys[i];
       if (MODE == 2) {
         y[rowg0 + i] = t;
-        if (deliver) vs_deliver<DIM>(hx, n0 + i / DIM, i % DIM, t);
       } else {
         const double uv = q == 0 ? pu[0] : q == 1 ? pu[1] : u[rowg0 + i];
         const double pv = MODE != 3 ? 0.0 : q == 0 ? pp[0] : q == 1 ? pp[1] : poly[rowg0 + i];
         const double yv = pc.cu * uv + pc.ct * t;
         y[rowg0 + i] = yv;
-        if (deliver) vs_deliver<DIM>(hx, n0 + i / DIM, i % DIM, yv);
         if (MODE == 3) poly[rowg0 + i] = pv + pc.cpu * uv + pc.cpy * yv;
       }
     }
     __syncwarp();
     if (lane == 0) mbar_arrive(empty + s);        // this warp is done with the stage (values, x, sums)
-  }
-  if (HALO && hx.push_seq) {
-    // every consumer warp of the grid checks out once its remote stores are fenced; the last one publishes the sequence
-    // number to the peers
-    __threadfence_system();
-    __syncwarp();
-    unsigned int prev = 0;
-    if (lane == 0) prev = atomicAdd(hx.counter, 1u);
-    prev = __shfl_sync(NSB_FULL, prev, 0);
-    if (prev == gridDim.x * (VS_GROUPS * VS_CONSUMERS) - 1) {
-      __threadfence_system();
-      if (lane < hx.npeers) {
-        volatile unsigned long long* f = hx.peer_flags[lane] + hx.my_rank;
-        *f = hx.push_seq;
-      }
-      if (lane == 0) *hx.counter = 0;
-      __threadfence_system();
-    }
-  }
-}
-
-template <int DIM> __device__ __forceinline__ void vs_deliver(const VsHalo& hx, int node, int comp, double v) {
-  for (int k = __ldg(hx.send_ptr + node); k < __ldg(hx.send_ptr + node + 1); ++k) {
-    const int2 d = __ldg(hx.send_dst + k);
-    hx.peer_arena[d.x][hx.y_off + d.y + comp] = v;
   }
 }
 

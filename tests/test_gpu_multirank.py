@@ -1,6 +1,6 @@
 """BASELINE config 3 ("mesh-3D-5 ... 1 vs 2 GPUs") as a -m gpu test: tools/gpu_multi.py under torchrun with one
-process per visible GPU (2, 4 or 8): peer-store halo (CUDA IPC over NVLink) fused into the streamed operator, the same
-halo as separate push / wait kernels, and the NCCL send/recv halo.  Skipped on a single-GPU box.
+process per visible GPU (2, 4 or 8): peer-store halo (CUDA IPC over NVLink, separate push / wait kernels) and the NCCL
+send/recv halo.  Skipped on a single-GPU box.
 
 Asserted per rank: pattern of the owned rows bit-exact against the oracle (reference cpp:256-273), A and b
 relative 1e-12 against the oracle AND bit-exact against a single-GPU assembly (SURVEY 8c pin 6), the
@@ -36,14 +36,14 @@ def _free_port():
     return p
 
 
-@pytest.mark.parametrize("fused,halo", [("1", "p2p"), ("0", "p2p"), ("0", "nccl")])
-def test_multi_gpu_matches_oracle_and_single_gpu(tmp_path, fused, halo):
+@pytest.mark.parametrize("halo", ["p2p", "nccl"])
+def test_multi_gpu_matches_oracle_and_single_gpu(tmp_path, halo):
     n = _ngpus()
     if n < 2:
         pytest.skip("needs >= 2 GPUs (run with gpurun --gpus 2)")
     world = 8 if n >= 8 else 4 if n >= 4 else 2
     out = str(tmp_path / "multi.json")
-    env = dict(os.environ, NSB200_FUSED_HALO=fused, NSB200_HALO=halo, OMP_NUM_THREADS="4")
+    env = dict(os.environ, NSB200_HALO=halo, OMP_NUM_THREADS="4")
     cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(world), "--master-addr", "127.0.0.1",
            "--master-port", str(_free_port()), os.path.join(ROOT, "tools", "gpu_multi.py"), "--json", out, "--lc", "0.05"]
     r = subprocess.run(cmd, env=env, capture_output=True, text=True, timeout=1500)
@@ -51,7 +51,7 @@ def test_multi_gpu_matches_oracle_and_single_gpu(tmp_path, fused, halo):
     s = json.load(open(out))
     keep = os.path.join(ROOT, "gpurun_out")
     if os.path.isdir(keep):
-        json.dump(s, open(os.path.join(keep, "multirank_n%d_fused%s_%s.json" % (world, fused, halo)), "w"), indent=1)
+        json.dump(s, open(os.path.join(keep, "multirank_n%d_%s.json" % (world, halo)), "w"), indent=1)
     assert s["world"] == world and len(s["ranks"]) == world
     assert sum(r_["rows"] for r_ in s["ranks"]) == s["n_dofs"]
     for r_ in s["ranks"]:

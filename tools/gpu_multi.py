@@ -135,7 +135,7 @@ def main():
     rec = dict(rank=rank, world=world, rows=int(nrows), cells=int(nc), pattern_ok=bool(okpat), A_relerr=float(errA),
                A_bitexact_vs_1gpu=bool(bitexact), b_relerr=float(errb), b_bitexact_vs_1gpu=b_bitexact,
                gmres_ok=bool(ok), gmres_its=int(it), gmres_its_1gpu=int(it1), tight_ok=bool(ok2), tight_its=int(it2),
-               field_relerr_vs_direct=ferr, slots_bitexact_vs_1gpu=slots_bitexact, fused=os.environ.get("NSB200_FUSED_HALO", "0"), halo=os.environ.get("NSB200_HALO", "p2p"))
+               field_relerr_vs_direct=ferr, slots_bitexact_vs_1gpu=slots_bitexact, halo=os.environ.get("NSB200_HALO", "p2p"))
     print("[rank %d/%d] " % (rank, world) + json.dumps(rec), flush=True)
     dist.barrier()
     dev.close()
@@ -178,7 +178,7 @@ def main():
         for src in pieces:
             piece = ET.parse(outdir + src).getroot().find("UnstructuredGrid/Piece")
             ncell += int(piece.get("NumberOfCells"))
-        summary = dict(world=world, partition=args.part, forcing=bool(args.forcing), forcing_source=bool(args.forcing_source), fused=os.environ.get("NSB200_FUSED_HALO", "0"), halo=os.environ.get("NSB200_HALO", "p2p"), mesh_cells=int(mesh.n_cells), n_dofs=int(N),
+        summary = dict(world=world, partition=args.part, forcing=bool(args.forcing), forcing_source=bool(args.forcing_source), halo=os.environ.get("NSB200_HALO", "p2p"), mesh_cells=int(mesh.n_cells), n_dofs=int(N),
                        ranks=recs, host_class_steps=steps, host_class_field_relerr=field, vtu_pieces=pieces, vtu_cells_total=ncell)
         print("[summary] " + json.dumps(summary), flush=True)
         if args.json:
