@@ -106,6 +106,17 @@ int nsb_set_solver_opts(nsb_handle h, const nsb_solver_opts* o);
 /* the options in effect (defaults resolved) */
 int nsb_get_solver_opts(nsb_handle h, nsb_solver_opts* out);
 
+/* Run state: what the library decides once and keeps for the rest of a run, so that a restarted run can carry it over.
+ *   cycle_disabled = 1 once the two-level velocity cycle has stalled: the single-level polynomial stays in charge.
+ * The flag is decided from the global iteration count, so it is the same on every rank; both calls act the same way on every
+ * rank.  nsb_set_solver_opts and nsb_upload_mesh reset it to 0, so on resume the order is: set the options, upload the mesh,
+ * then nsb_set_run_state.  Errors before nsb_upload_mesh.
+ * Not part of the state: the solve counter and the cached polynomial roots.  With the default poly_refresh = 1 the velocity
+ * preconditioner is rebuilt at every solve, so they carry nothing; with poly_refresh > 1 a resumed run rebuilds the
+ * polynomial at its first solve, and its continuation is not bit-identical to the uninterrupted run. */
+int nsb_get_run_state(nsb_handle h, int32_t* cycle_disabled);
+int nsb_set_run_state(nsb_handle h, int32_t cycle_disabled);
+
 enum {
   NSB_SOLUTION_OLD = 0,      /* solution_old        u^n                (hpp:578)           */
   NSB_SOLUTION_OLD_OLD = 1,  /* solution_old_old    u^{n-1}            (hpp:587)           */

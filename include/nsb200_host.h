@@ -33,6 +33,9 @@ typedef struct nsh_options {
   int32_t partitioner;       /* cells -> ranks: 0 contiguous chunks (default), 1 METIS on the face-dual graph (cpp:56) */
   int32_t test_fail_solves;  /* test hook: report the next k linear solves as not converged (drives the retry /
                                 fallback paths of run(), cpp:1174-1198, 1223-1286); 0 in production           */
+  int32_t restart_every;     /* run(): write a restart file after every step whose number is a multiple of this, and after
+                                its last step; 0 = never                                                       */
+  const char* restart_file;  /* where run() writes it; NULL = output_dir + "restart.nsb"                       */
 } nsh_options;
 
 typedef struct nsh_step_info {
@@ -49,6 +52,12 @@ const char* nsh_last_error(void);
 int nsh_create(const char* test_case, const char* mesh_file, const nsh_options* opt, nsh_handle* out);
 void nsh_destroy(nsh_handle h);
 int nsh_initialize(nsh_handle h);                        /* setup() + initial condition (cpp:1045-1071) */
+/* Restart files (NavierStokes::save_restart / resume, DESIGN.md section 12).  nsh_save_restart: call on every rank after a
+ * step; rank 0 writes the file atomically (path.tmp, fsync, rename).  nsh_resume: in place of nsh_initialize; fails, naming
+ * the field, when the file does not belong to this mesh / test case / dt, or is truncated or corrupt.  Set the forcing again
+ * before stepping: it is not stored. */
+int nsh_resume(nsh_handle h, const char* path);
+int nsh_save_restart(nsh_handle h, const char* path);
 int nsh_step(nsh_handle h, nsh_step_info* info);         /* one time step of run() (cpp:1074-1322)      */
 int nsh_run(nsh_handle h);                               /* run()                                        */
 int nsh_get_sizes(nsh_handle h, int64_t* n_u, int64_t* n_p, int64_t* n_cells, int64_t* n_vertices);

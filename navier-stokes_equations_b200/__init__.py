@@ -162,6 +162,16 @@ class Device:
         self._ck(lib().nsb_get_solver_opts(self.h, C.byref(o)))
         return {k: getattr(o, k) for k, _ in NsbSolverOpts._fields_}
 
+    def run_state(self):
+        """What the library decided once and keeps for the run (nsb_get_run_state): dict(cycle_disabled).  Needs a mesh."""
+        cd = C.c_int32()
+        self._ck(lib().nsb_get_run_state(self.h, C.byref(cd)))
+        return dict(cycle_disabled=bool(cd.value))
+
+    def set_run_state(self, cycle_disabled):
+        """Restore a saved run state (nsb_set_run_state) after set_solver_opts and upload_mesh, which reset it."""
+        self._ck(lib().nsb_set_run_state(self.h, C.c_int32(int(cycle_disabled))))
+
     def set_vector(self, which, v):
         v = np.ascontiguousarray(v, np.float64)
         assert v.shape[0] == self.n_dofs
@@ -405,7 +415,8 @@ _hostlib = None
 class NshOptions(C.Structure):
     _fields_ = [("device", C.c_int32), ("rank", C.c_int32), ("nranks", C.c_int32), ("nccl_unique_id", C.c_void_p),
                 ("write_vtu", C.c_int32), ("verbose", C.c_int32), ("gmres_tolerance", C.c_double), ("deltat", C.c_double),
-                ("max_steps", C.c_int32), ("output_dir", C.c_char_p), ("solver", NsbSolverOpts), ("partitioner", C.c_int32), ("test_fail_solves", C.c_int32)]
+                ("max_steps", C.c_int32), ("output_dir", C.c_char_p), ("solver", NsbSolverOpts), ("partitioner", C.c_int32), ("test_fail_solves", C.c_int32),
+                ("restart_every", C.c_int32), ("restart_file", C.c_char_p)]
 
 
 class NshStepInfo(C.Structure):
@@ -446,12 +457,15 @@ class HostSolver:
     """NavierStokes<dim>(TestCases::make_<case>(mesh_file)) driven through the C facade."""
 
     def __init__(self, case, mesh_file, device=0, rank=0, nranks=1, nccl_unique_id=None, write_vtu=False, verbose=False,
-                 gmres_tolerance=0.0, deltat=0.0, output_dir=None, solver_opts=None, test_fail_solves=0, partitioner=0):
+                 gmres_tolerance=0.0, deltat=0.0, output_dir=None, solver_opts=None, test_fail_solves=0, partitioner=0,
+                 restart_every=0, restart_file=None):
         L = hostlib()
         self._uid = C.create_string_buffer(nccl_unique_id, 128) if nccl_unique_id else None
         self._outdir = output_dir.encode() if output_dir else None
+        self._restart_file = restart_file.encode() if restart_file else None
         o = NshOptions(device, rank, nranks, C.cast(self._uid, C.c_void_p) if self._uid else None, int(write_vtu),
-                       int(verbose), gmres_tolerance, deltat, -1, self._outdir, solver_opts or NsbSolverOpts(), partitioner, test_fail_solves)
+                       int(verbose), gmres_tolerance, deltat, -1, self._outdir, solver_opts or NsbSolverOpts(), partitioner, test_fail_solves,
+                       restart_every, self._restart_file)
         self.h = C.c_void_p()
         if L.nsh_create(case.encode(), mesh_file.encode(), C.byref(o), C.byref(self.h)) != 0:
             raise NsbError(L.nsh_last_error().decode())
@@ -465,6 +479,19 @@ class HostSolver:
 
     def initialize(self):
         self._ck(hostlib().nsh_initialize(self.h))
+        self._sizes()
+
+    def resume(self, path):
+        """In place of initialize(): continue the run saved in `path` by save_restart (same mesh, test case and dt; the
+        forcing is not stored, set it before stepping).  Raises NsbError naming the mismatch, or for a truncated / corrupt file."""
+        self._ck(hostlib().nsh_resume(self.h, os.fsencode(path)))
+        self._sizes()
+
+    def save_restart(self, path):
+        """Write everything the time loop carries to the next step to `path` (call on every rank after a step; rank 0 writes)."""
+        self._ck(hostlib().nsh_save_restart(self.h, os.fsencode(path)))
+
+    def _sizes(self):
         v = [C.c_int64() for _ in range(4)]
         self._ck(hostlib().nsh_get_sizes(self.h, *[C.byref(x) for x in v]))
         self.n_u, self.n_p, self.n_cells, self.n_vertices = [x.value for x in v]

@@ -2865,6 +2865,20 @@ int nsb_get_solver_opts(nsb_handle c, nsb_solver_opts* o) {
   return 0;
 }
 
+int nsb_get_run_state(nsb_handle c, int32_t* cycle_disabled) {
+  if (!c || !cycle_disabled) return -1;
+  if (!c->have_mesh) return fail(c, "nsb_get_run_state: no mesh uploaded");
+  *cycle_disabled = c->cycle_disabled ? 1 : 0;
+  return 0;
+}
+
+int nsb_set_run_state(nsb_handle c, int32_t cycle_disabled) {
+  if (!c) return -1;
+  if (!c->have_mesh) return fail(c, "nsb_set_run_state: no mesh uploaded (order: solver options, mesh, run state)");
+  c->cycle_disabled = cycle_disabled != 0;
+  return 0;
+}
+
 int nsb_launch_count(nsb_handle c, int64_t* n) {
   if (!c) return -1;
   *n = c->launches;

@@ -106,6 +106,8 @@ int nsh_create(const char* test_case, const char* mesh_file, const nsh_options* 
     ro.solver = o->solver;
     ro.partitioner = o->partitioner;
     ro.test_fail_solves = o->test_fail_solves;
+    ro.restart_every = o->restart_every;
+    if (o->restart_file) ro.restart_file = o->restart_file;
     dt = o->deltat;
   }
   auto h = std::make_unique<nsh_solver>();
@@ -122,6 +124,22 @@ void nsh_destroy(nsh_handle h) { delete h; }
 int nsh_initialize(nsh_handle h) {
   NSH_TRY
   if (h->dim == 2) h->s2->initialize(); else h->s3->initialize();
+  return 0;
+  NSH_CATCH
+}
+
+int nsh_resume(nsh_handle h, const char* path) {
+  if (!h || !path) { g_err = "null argument"; return -1; }
+  NSH_TRY
+  if (h->dim == 2) h->s2->resume(path); else h->s3->resume(path);
+  return 0;
+  NSH_CATCH
+}
+
+int nsh_save_restart(nsh_handle h, const char* path) {
+  if (!h || !path) { g_err = "null argument"; return -1; }
+  NSH_TRY
+  if (h->dim == 2) h->s2->save_restart(path); else h->s3->save_restart(path);
   return 0;
   NSH_CATCH
 }

@@ -1,7 +1,9 @@
 // Driver with the same role as the reference's src/main.cpp:3-46, except that the test case and
 // mesh are chosen on the command line instead of by editing the source:
 //   navier_stokes <test case> <mesh file> [--steps N] [--no-vtu] [--tol X] [--device D]
-//                 [--forcing FILE.cu [--forcing-params a,b,...]]
+//                 [--forcing FILE.cu [--forcing-params a,b,...]] [--restart-every K] [--restart-file F] [--resume F]
+// --restart-every: write a restart file (default ./restart.nsb, --restart-file) after every K-th step and after the last one;
+// --resume: continue the run saved in F instead of starting at t = 0 (--steps then counts the steps of this invocation).
 // --forcing: the forcing term as CUDA source evaluated on the GPU (DeviceForcing, include/nsb200.h nsb_set_forcing_source),
 // with up to 16 parameters.
 #include <cstdlib>
@@ -50,7 +52,7 @@ int main(int argc, char* argv[]) {
   try {
     if (argc < 3) {
       std::cerr << "usage: " << argv[0] << " <2D-1|2D-2|2D-3|3D-1Z|3D-2Z|3D-3Z> <mesh.msh|mesh.bin> [--steps N] [--no-vtu] [--tol X] [--device D]"
-                << " [--forcing FILE.cu [--forcing-params a,b,...]]" << std::endl;
+                << " [--forcing FILE.cu [--forcing-params a,b,...]] [--restart-every K] [--restart-file F] [--resume F]" << std::endl;
       return 2;
     }
     const std::string tc_name = argv[1], mesh = argv[2];
@@ -62,6 +64,9 @@ int main(int argc, char* argv[]) {
       else if (!std::strcmp(argv[i], "--device") && i + 1 < argc) opt.device = std::atoi(argv[++i]);
       else if (!std::strcmp(argv[i], "--forcing") && i + 1 < argc) forcing_src = read_file(argv[++i]);
       else if (!std::strcmp(argv[i], "--forcing-params") && i + 1 < argc) forcing_params = parse_list(argv[++i]);
+      else if (!std::strcmp(argv[i], "--restart-every") && i + 1 < argc) opt.restart_every = std::atoi(argv[++i]);
+      else if (!std::strcmp(argv[i], "--restart-file") && i + 1 < argc) opt.restart_file = argv[++i];
+      else if (!std::strcmp(argv[i], "--resume") && i + 1 < argc) opt.resume_file = argv[++i];
     }
     if (!forcing_params.empty() && forcing_src.empty()) throw std::runtime_error("--forcing-params needs --forcing FILE.cu");
     if (tc_name == "2D-1") run(TestCases::make_2D_1(mesh), opt);

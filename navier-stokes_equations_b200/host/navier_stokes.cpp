@@ -3,7 +3,10 @@
 // hot path is a call into the CUDA library through the C ABI (include/nsb200.h).
 #include "navier_stokes.hpp"
 
+#include <unistd.h>
+
 #include <algorithm>
+#include <cerrno>
 #include <cstdio>
 #include <cstring>
 #include <iomanip>
@@ -17,6 +20,46 @@ namespace {
 struct NullBuf : std::streambuf { int overflow(int c) override { return c; } };
 NullBuf g_nullbuf;
 std::ostream g_null(&g_nullbuf);
+
+// ---- restart files (layout above NavierStokes::save_restart)
+static_assert(__BYTE_ORDER__ == __ORDER_LITTLE_ENDIAN__, "restart files are written and read as little-endian memory images");
+constexpr char kRestartMagic[8] = {'N', 'S', 'B', 'R', 'S', 'T', '0', '1'};
+constexpr uint64_t kFnvOffset = 14695981039346656037ull, kFnvPrime = 1099511628211ull;
+
+uint64_t fnv1a(const void* p, size_t n, uint64_t h = kFnvOffset) {
+  const unsigned char* b = static_cast<const unsigned char*>(p);
+  for (size_t i = 0; i < n; ++i) { h ^= b[i]; h *= kFnvPrime; }
+  return h;
+}
+
+struct RestartWriter {                 // writes to f and hashes what it wrote
+  std::FILE* f;
+  const std::string& path;
+  uint64_t hash = kFnvOffset;
+  void raw(const void* p, size_t n) {
+    if (std::fwrite(p, 1, n, f) != n) throw std::runtime_error("cannot write restart file " + path + ": " + std::strerror(errno));
+    hash = fnv1a(p, n, hash);
+  }
+  template <class T> void put(T v) { raw(&v, sizeof v); }
+};
+
+struct RestartReader {                 // bounds-checked reads from the file image
+  const std::vector<char>& buf;
+  size_t pos;
+  const std::string& where;
+  void raw(void* p, size_t n) {
+    if (n > buf.size() - pos) throw std::runtime_error(where + "truncated inside its header (" + std::to_string(buf.size()) + " bytes)");
+    std::memcpy(p, buf.data() + pos, n);
+    pos += n;
+  }
+  template <class T> T get() { T v; raw(&v, sizeof v); return v; }
+};
+
+std::string exact(double v) {
+  std::ostringstream s;
+  s << std::setprecision(17) << v;
+  return s.str();
+}
 }  // namespace
 
 template <int dim>
@@ -723,12 +766,188 @@ template <int dim> StepInfo NavierStokes<dim>::advance() {                      
   return info;
 }
 
+// ------------------------------------------------------------------------------------ restart files
+// One file, little-endian, vectors in the global DoF numbering (so it does not depend on the partition):
+//   "NSBRST01" | i32 dim | i64 n_u, n_p, n_cells, n_vertices | u64 mesh_hash() | u32 length + bytes of the test case name |
+//   f64 Re, U_m, dt | i32 time scheme (0 BE, 1 CN), nonlinear method (0 Newton, 1 linearised), use_supg | f64 T |
+//   f64 time | i64 time_step_no | i32 first_step, second_step, cycle_disabled (nsb_get_run_state) |
+//   f64 current_solution[n], solution_old[n], solution_old_old[n] (n = n_u + n_p) |
+//   u64 FNV-1a of everything between the magic and this checksum
+template <int dim> uint64_t NavierStokes<dim>::mesh_hash() const {
+  uint64_t h = fnv1a(mesh.points.data(), mesh.points.size() * sizeof(double));
+  h = fnv1a(mesh.cells.data(), mesh.cells.size() * sizeof(uint32_t), h);
+  for (const auto& b : bfaces) {                   // after the geometric id fallback of setup()
+    const int64_t cell = b.cell;
+    const int32_t face = b.face, id = b.id;
+    h = fnv1a(&cell, sizeof cell, h);
+    h = fnv1a(&face, sizeof face, h);
+    h = fnv1a(&id, sizeof id, h);
+  }
+  return h;
+}
+
+template <int dim> void NavierStokes<dim>::save_restart(const std::string& path) const {
+  if (!dev) throw std::runtime_error("save_restart: the solver is not set up (call initialize() or resume() first)");
+  int32_t cycle_disabled = 0;
+  ck(nsb_get_run_state(dev, &cycle_disabled), "nsb_get_run_state");
+  if (mpi_rank != 0) return;                       // the vectors are global on every rank
+  const std::string tmp = path + ".tmp";
+  std::FILE* f = std::fopen(tmp.c_str(), "wb");
+  if (!f) throw std::runtime_error("cannot write restart file " + tmp + ": " + std::strerror(errno));
+  try {
+    if (std::fwrite(kRestartMagic, 1, sizeof kRestartMagic, f) != sizeof kRestartMagic)
+      throw std::runtime_error("cannot write restart file " + tmp + ": " + std::strerror(errno));
+    RestartWriter w{f, tmp};
+    w.put<int32_t>(dim);
+    w.put<int64_t>(dof_handler.n_u);
+    w.put<int64_t>(dof_handler.n_p);
+    w.put<int64_t>(mesh.n_cells());
+    w.put<int64_t>(mesh.n_vertices());
+    w.put<uint64_t>(mesh_hash());
+    w.put<uint32_t>((uint32_t)case_name.size());
+    w.raw(case_name.data(), case_name.size());
+    w.put<double>(Re);
+    w.put<double>(U_m);
+    w.put<double>(deltat);
+    w.put<int32_t>(time_scheme == TimeScheme::CrankNicolson ? 1 : 0);
+    w.put<int32_t>(nonlinear_method == NonlinearMethod::Linearized ? 1 : 0);
+    w.put<int32_t>(use_supg ? 1 : 0);
+    w.put<double>(T);
+    w.put<double>(time);
+    w.put<int64_t>(time_step_no);
+    w.put<int32_t>(first_step ? 1 : 0);
+    w.put<int32_t>(second_step ? 1 : 0);
+    w.put<int32_t>(cycle_disabled);
+    for (const auto* v : {&current_solution, &solution_old, &solution_old_old}) w.raw(v->data(), v->size() * sizeof(double));
+    const uint64_t sum = w.hash;
+    if (std::fwrite(&sum, 1, sizeof sum, f) != sizeof sum || std::fflush(f) != 0 || ::fsync(fileno(f)) != 0)
+      throw std::runtime_error("cannot write restart file " + tmp + ": " + std::strerror(errno));
+  } catch (...) {
+    std::fclose(f);
+    std::remove(tmp.c_str());
+    throw;
+  }
+  if (std::fclose(f) != 0) {
+    std::remove(tmp.c_str());
+    throw std::runtime_error("cannot write restart file " + tmp + ": " + std::strerror(errno));
+  }
+  if (std::rename(tmp.c_str(), path.c_str()) != 0)
+    throw std::runtime_error("cannot rename " + tmp + " to " + path + ": " + std::strerror(errno));
+}
+
+template <int dim> void NavierStokes<dim>::resume(const std::string& path) {
+  // 1. the whole file: magic, size against its header, checksum
+  const std::string where = "restart file " + path + ": ";
+  std::vector<char> buf;
+  {
+    std::ifstream in(path, std::ios::binary | std::ios::ate);
+    if (!in) throw std::runtime_error("cannot open restart file " + path);
+    buf.resize((size_t)in.tellg());
+    in.seekg(0);
+    if (!in.read(buf.data(), (std::streamsize)buf.size())) throw std::runtime_error("cannot read restart file " + path);
+  }
+  if (buf.size() < sizeof kRestartMagic || std::memcmp(buf.data(), kRestartMagic, sizeof kRestartMagic) != 0)
+    throw std::runtime_error(where + "not a restart file (no NSBRST01 magic)");
+  RestartReader r{buf, sizeof kRestartMagic, where};
+  const int32_t f_dim = r.get<int32_t>();
+  const int64_t f_nu = r.get<int64_t>(), f_np = r.get<int64_t>(), f_nc = r.get<int64_t>(), f_nv = r.get<int64_t>();
+  const uint64_t f_hash = r.get<uint64_t>();
+  const uint32_t name_len = r.get<uint32_t>();
+  if (name_len > 256) throw std::runtime_error(where + "corrupt header (test case name of " + std::to_string(name_len) + " bytes)");
+  std::string f_case(name_len, '\0');
+  r.raw(f_case.data(), name_len);
+  const double f_Re = r.get<double>(), f_Um = r.get<double>(), f_dt = r.get<double>();
+  const int32_t f_scheme = r.get<int32_t>(), f_method = r.get<int32_t>(), f_supg = r.get<int32_t>();
+  r.get<double>();                                  // T: a resumed run may go further than the saved one
+  const double f_time = r.get<double>();
+  const int64_t f_step = r.get<int64_t>();
+  const int32_t f_first = r.get<int32_t>(), f_second = r.get<int32_t>(), f_cycle = r.get<int32_t>();
+  if (f_nu < 0 || f_np < 0 || f_nu + f_np > (int64_t(1) << 40))
+    throw std::runtime_error(where + "corrupt header (n_u = " + std::to_string(f_nu) + ", n_p = " + std::to_string(f_np) + ")");
+  const size_t n = (size_t)(f_nu + f_np), vec_pos = r.pos, expected = vec_pos + 3 * n * sizeof(double) + sizeof(uint64_t);
+  if (buf.size() != expected)
+    throw std::runtime_error(where + (buf.size() < expected ? "truncated: " : "too long: ") + std::to_string(buf.size()) +
+                             " bytes, its header describes " + std::to_string(expected));
+  uint64_t stored;
+  std::memcpy(&stored, buf.data() + buf.size() - sizeof stored, sizeof stored);
+  if (fnv1a(buf.data() + sizeof kRestartMagic, buf.size() - sizeof kRestartMagic - sizeof stored) != stored)
+    throw std::runtime_error(where + "checksum mismatch (the file is corrupt)");
+
+  // 2. the solver as initialize() sets it up
+  setup();
+
+  // 3. the file must describe this solver; nothing below is changed before every field is checked
+  auto check = [&](bool same, const std::string& field, const std::string& in_file, const std::string& here) {
+    if (!same) throw std::runtime_error(where + field + " is " + in_file + " in the file but " + here + " in this solver");
+  };
+  const std::string schemes[2] = {to_string(TimeScheme::BackwardEuler), to_string(TimeScheme::CrankNicolson)};
+  const std::string methods[2] = {to_string(NonlinearMethod::Newton), to_string(NonlinearMethod::Linearized)};
+  const int scheme = time_scheme == TimeScheme::CrankNicolson ? 1 : 0;
+  const int method = nonlinear_method == NonlinearMethod::Linearized ? 1 : 0;
+  check(f_dim == dim, "dim", std::to_string(f_dim), std::to_string(dim));
+  check(f_nu == dof_handler.n_u, "n_u (velocity DoFs)", std::to_string(f_nu), std::to_string(dof_handler.n_u));
+  check(f_np == dof_handler.n_p, "n_p (pressure DoFs)", std::to_string(f_np), std::to_string(dof_handler.n_p));
+  check(f_nc == mesh.n_cells(), "n_cells", std::to_string(f_nc), std::to_string(mesh.n_cells()));
+  check(f_nv == mesh.n_vertices(), "n_vertices", std::to_string(f_nv), std::to_string(mesh.n_vertices()));
+  const uint64_t hash = mesh_hash();
+  char hf[24], hh[24];
+  std::snprintf(hf, sizeof hf, "%016llx", (unsigned long long)f_hash);
+  std::snprintf(hh, sizeof hh, "%016llx", (unsigned long long)hash);
+  check(f_hash == hash, "the mesh hash (vertices, cells, boundary ids)", hf, hh);
+  check(f_case == case_name, "the test case", "'" + f_case + "'", "'" + case_name + "'");
+  check(f_Re == Re, "Re", exact(f_Re), exact(Re));
+  check(f_Um == U_m, "U_m", exact(f_Um), exact(U_m));
+  check(f_dt == deltat, "the time step dt", exact(f_dt), exact(deltat));
+  check(f_scheme == scheme, "the time scheme", f_scheme == 0 || f_scheme == 1 ? schemes[f_scheme] : std::to_string(f_scheme), schemes[scheme]);
+  check(f_method == method, "the nonlinear method", f_method == 0 || f_method == 1 ? methods[f_method] : std::to_string(f_method), methods[method]);
+  check((f_supg != 0) == use_supg, "use_supg", std::to_string(f_supg), std::to_string((int)use_supg));
+
+  // 4. the state the time loop carries from one step to the next
+  time = f_time;
+  time_step_no = (unsigned int)f_step;
+  first_step = f_first != 0;
+  second_step = f_second != 0;
+  for (auto* v : {&current_solution, &solution_old, &solution_old_old}) {
+    std::memcpy(v->data(), buf.data() + r.pos, n * sizeof(double));
+    r.pos += n * sizeof(double);
+  }
+  solution_owned = current_solution;                // as advance() leaves them
+  solution = current_solution;
+  ck(nsb_set_run_state(dev, f_cycle), "nsb_set_run_state");
+
+  // 5. forces.txt: keep the header and the first time_step_no rows (a run that died after this file was written has
+  //    appended more), append from there
+  if (mpi_rank == 0) {
+    const std::string fp = options.output_dir + "forces.txt";
+    size_t keep = 0;
+    {
+      std::ifstream in(fp, std::ios::binary);
+      std::string line;
+      for (unsigned int rows = 0; in && rows <= time_step_no && std::getline(in, line); ++rows) keep += line.size() + 1;
+    }
+    if (keep > 0) {
+      if (::truncate(fp.c_str(), (off_t)keep) != 0) throw std::runtime_error("cannot truncate " + fp + ": " + std::strerror(errno));
+      forces_file.open(fp, std::ios::app);
+    } else {                                        // no file, or an empty one
+      forces_file.open(fp);
+      forces_file << "Time\tCd\tCl\tDeltaP" << std::endl;
+    }
+  }
+
+  // 6. no output(0): the VTU numbering continues at time_step_no + 1
+  pcout << "Resuming from " << path << ": step " << time_step_no << ", t=" << time << std::endl;
+}
+
 template <int dim> void NavierStokes<dim>::run() {                              // cpp:1044-1327
-  initialize();
+  if (options.resume_file.empty()) initialize();
+  else resume(options.resume_file);
+  const std::string restart_path = options.restart_file.empty() ? options.output_dir + "restart.nsb" : options.restart_file;
   int steps = 0;
   while (time < T) {
     advance();
-    if (options.max_steps >= 0 && ++steps >= options.max_steps) break;
+    const bool last = (options.max_steps >= 0 && ++steps >= options.max_steps) || !(time < T);
+    if (options.restart_every > 0 && (time_step_no % (unsigned int)options.restart_every == 0 || last)) save_restart(restart_path);
+    if (last) break;
   }
   pcout << "===============================================" << std::endl;
   pcout << "Simulation complete." << std::endl;

@@ -100,6 +100,10 @@ struct RunOptions {
   int partitioner = 0;            // cells -> ranks: 0 = contiguous chunks, 1 = METIS on the face-dual graph (partition_cells, mesh.hpp)
   int test_fail_solves = 0;       // test hook: the next k linear solves are REPORTED as not converged (their result is kept,
                                   // as the reference keeps the iterate of a failed GMRES) -> drives run()'s retry / fallback paths
+  int restart_every = 0;          // run(): save_restart after every step whose number is a multiple of this, and after the
+                                  // last step of the invocation (0 = off)
+  std::string restart_file;       // where run() saves; empty = output_dir + "restart.nsb"
+  std::string resume_file;        // run() resumes from this file instead of initialize() (empty = initialize())
 };
 
 struct StepInfo {
@@ -123,7 +127,9 @@ public:
   explicit NavierStokes(const BenchmarkTestCase<dim>& tc, const RunOptions& opt = RunOptions())
     : NavierStokes(tc.mesh_file, tc.degree_velocity, tc.degree_pressure, tc.deltat, tc.T, tc.Re, tc.U_m, tc.time_scheme,
                    tc.nonlinear_method, tc.inlet_velocity, tc.dirichlet_bc, tc.forcing_term, tc.initial_condition,
-                   tc.use_supg, opt) {}
+                   tc.use_supg, opt) {
+    case_name = tc.name;
+  }
 
   NavierStokes(const std::string& mesh_file_name_, const unsigned int& degree_velocity_,
                const unsigned int& degree_pressure_, const double deltat_, const double T_, const double Re_,
@@ -152,6 +158,14 @@ public:
   // ---- additions for drivers / tests (no counterpart in the reference) ----
   void initialize();                 // setup() + initial condition, as the head of run() (cpp:1045-1068)
   StepInfo advance();                // one pass of the while loop body of run() (cpp:1074-1322)
+  // Restart files (DESIGN.md section 12).  save_restart: call on every rank after advance() returns; rank 0 writes
+  // path + ".tmp", flushes, fsyncs and renames it to path, so an earlier file survives a crash mid-write.  resume: in place
+  // of initialize(); checks the file against this solver (mesh, test case, Re, U_m, dt, scheme, method, SUPG) and throws,
+  // naming the field, before it changes anything; continues forces.txt after its first time_step_no rows and the VTU
+  // numbering at time_step_no + 1.  With the same options and forcing the continuation is bit-identical to the run that
+  // was never interrupted (not with poly_refresh > 1).  The forcing term is code, not state: set it again before stepping.
+  void save_restart(const std::string& path) const;
+  void resume(const std::string& path);
   const std::vector<double>& current() const { return current_solution; }
   const DofHandler& dofs() const { return dof_handler; }
   const Mesh& grid() const { return mesh; }
@@ -165,6 +179,7 @@ protected:
   std::ostream& pcout;
   bool pcout_active;
   const std::string mesh_file_name;
+  std::string case_name;               // BenchmarkTestCase::name, written to restart files (empty without a test case)
   const unsigned int degree_velocity, degree_pressure;
   Mesh mesh;
   double Re;
@@ -226,6 +241,7 @@ protected:
   void push_params(bool first_order);
   void update_forcing();
   void build_system_constraints();
+  uint64_t mesh_hash() const;          // FNV-1a of the vertices, cell vertex lists and boundary faces with their ids
   void ck(int rc, const char* what) const;
   std::function<double(const double*, int)> eval(const std::shared_ptr<Function<dim>>& f) const;
 };

@@ -6,9 +6,11 @@ the tight-tolerance solve against a sparse direct solve, the iteration count at 
 samples it at its own local cells' quadrature points (owned + ghost layer), the oracle at its own, and the host class
 takes it through HostSolver.set_forcing.  --forcing-source does the same with the force given as CUDA source: every rank
 compiles it and evaluates it on the device at its own local cells (ghost layer included), and the slots are compared bit
-for bit with the single-GPU ones, cell by cell.
-  python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/gpu_multi.py [--json out.json] [--forcing | --forcing-source]
-tests/test_gpu_multirank.py and tests/test_gpu_forcing.py run this under pytest and assert on the JSON."""
+for bit with the single-GPU ones, cell by cell.  --restart checks restart files instead (and nothing else): the ranks save
+at step 2 and go on to step 4; fresh solvers on the same ranks resume the file and must repeat steps 3-4 bit for bit on every
+rank; one GPU resuming the same file must follow within the tight-tolerance bars (the file is in the global numbering).
+  python -m torch.distributed.run --nproc-per-node 2 --master-addr 127.0.0.1 tools/gpu_multi.py [--json out.json] [--forcing | --forcing-source | --restart]
+tests/test_gpu_multirank.py, tests/test_gpu_forcing.py and tests/test_gpu_restart.py run this under pytest and assert on the JSON."""
 import argparse
 import json
 import os
@@ -38,10 +40,15 @@ def main():
     ap.add_argument("--part", default="chunks", help="cell partition: chunks (contiguous) or metis (face-dual graph, like the reference)")
     ap.add_argument("--forcing", action="store_true", help="assemble and step with a non-zero body force")
     ap.add_argument("--forcing-source", action="store_true", help="the same body force as CUDA source evaluated on each GPU")
+    ap.add_argument("--restart", action="store_true", help="check save_restart / resume on these ranks and on one GPU")
     args = ap.parse_args()
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ["LOCAL_RANK"])
     torch.cuda.set_device(local)
     dist.init_process_group("nccl", device_id=torch.device("cuda", local))
+    if args.restart:
+        restart_main(args, rank, world, local)
+        dist.destroy_process_group()
+        return
     holder = [nsb.Device.comm_unique_id() if rank == 0 else None]
     dist.broadcast_object_list(holder, src=0)
     mesh = meshgen.mesh_3d(lc_cyl=args.lc, lc_global=0.15)
@@ -186,6 +193,70 @@ def main():
                 json.dump(summary, f, indent=1)
     dist.barrier()
     dist.destroy_process_group()
+
+
+def restart_main(args, rank, world, local):
+    """NavierStokes<3>(make_3D_2Z) on `world` GPUs at gmres_tolerance 1e-12: save at step 2, go on to step 4; fresh solvers
+    resume and repeat steps 3-4; one GPU resumes the same file."""
+    mesh = meshgen.mesh_3d(lc_cyl=args.lc, lc_global=0.15)
+    tmp = [tempfile.mkdtemp(prefix="nsb_restart_") if rank == 0 else None]
+    dist.broadcast_object_list(tmp, src=0)
+    base = tmp[0] + "/"
+    dirs = {k: base + k + "/" for k in ("a", "b", "one")}
+    if rank == 0:
+        for d in dirs.values():
+            os.makedirs(d)
+    path = base + "mesh_%d.bin" % rank
+    msh.write_bin(path, mesh)
+    restart = base + "restart.nsb"
+    skip = ("wall_seconds", "forcing_seconds")
+
+    def solver(outdir, nranks=world):
+        uid = [nsb.Device.comm_unique_id() if rank == 0 and nranks > 1 else None]
+        if nranks > 1:
+            dist.broadcast_object_list(uid, src=0)
+        return nsb.HostSolver("3D-2Z", path, device=local, rank=rank if nranks > 1 else 0, nranks=nranks, nccl_unique_id=uid[0],
+                              gmres_tolerance=1e-12, output_dir=outdir)
+
+    def steps(s, n):
+        return [{k: v for k, v in s.step().items() if k not in skip} for _ in range(n)]
+
+    dist.barrier()
+    a = solver(dirs["a"])
+    a.initialize()
+    steps(a, 2)
+    a.save_restart(restart)
+    dist.barrier()                                   # rank 0 has renamed the file into place
+    infos_a = steps(a, 2)
+    xa = a.solution()
+    a.close()
+    b = solver(dirs["b"])
+    b.resume(restart)
+    infos_b = steps(b, 2)
+    xb = b.solution()
+    b.close()
+    rec = dict(rank=rank, solution_bitexact=bool(xa.tobytes() == xb.tobytes()), steps_equal=bool(infos_a == infos_b))
+    print("[rank %d/%d] " % (rank, world) + json.dumps(rec), flush=True)
+    recs = [None] * world
+    dist.all_gather_object(recs, rec)
+    if rank == 0:
+        one = solver(dirs["one"], nranks=1)
+        one.resume(restart)
+        infos_1 = steps(one, 2)
+        x1 = one.solution()
+        one.close()
+        rows = lambda d: open(d + "forces.txt").read().strip().split("\n")[1:]
+        field = float(np.linalg.norm(x1 - xa) / np.linalg.norm(xa))
+        force = max(abs(i1[k] - ia[k]) / max(abs(ia[k]), 1e-300) if k != "cl" or abs(ia[k]) > 1e-10 else abs(i1[k] - ia[k])
+                    for i1, ia in zip(infos_1, infos_a) for k in ("cd", "cl", "dp"))
+        summary = dict(world=world, mesh_cells=int(mesh.n_cells), ranks=recs, forces_rows_equal=rows(dirs["a"])[2:] == rows(dirs["b"]),
+                       one_gpu_field_relerr=field, one_gpu_force_relerr=float(force), one_gpu_gmres=[i["gmres_iterations"] for i in infos_1],
+                       gmres=[i["gmres_iterations"] for i in infos_a])
+        print("[summary] " + json.dumps(summary), flush=True)
+        if args.json:
+            with open(args.json, "w") as f:
+                json.dump(summary, f, indent=1)
+    dist.barrier()
 
 
 if __name__ == "__main__":
